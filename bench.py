@@ -13,6 +13,8 @@ scaling).  Rank 0 prints ONE JSON line.  The same line carries
   ik            IK frame-iterations/s of the batched MoSh step (configs[2]-shaped) when available
   cpu_baseline  the reference's own libtorch CPU implementation (oracle/_ref) on this box's host cores
 `--impl reference` times only that CPU implementation and prints the line with "impl": "reference".
+`--dump-outputs DIR` writes what the last timed step computed (see DUMP_FRAMES) as DIR/<name>.npy, so that two builds
+can be compared output for output: the inputs are seeded and identical from run to run.
 """
 from __future__ import annotations
 
@@ -35,6 +37,9 @@ VERTS = 6890
 BYTES_FUSED = VERTS * 3 * 4 + (25 * 3 + 10) * 4  # vertices out + theta, beta in
 BYTES_LBS = 2 * VERTS * 3 * 4 + 24 * 12 * 4  # rest in + vertices out + 24 transforms
 FLOPS_BLEND = 2 * 218 * VERTS * 3  # pose (207) + shape (10) + template (1) contraction
+# --dump-outputs: vertices and joints of a fixed, seeded sample of this many frames of rank 0's batch (42 MB as float32;
+# all 4096 frames would be 340 MB)
+DUMP_FRAMES = 512
 
 
 def measured_peaks():
@@ -234,7 +239,14 @@ def main():
     ap.add_argument("--ik-frames-total", type=int, default=0,
                     help="BASELINE configs[4]: total mocap frames of the IK leg, sharded over the ranks as contiguous "
                          "blocks (default 0 = 16384 frames per GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the vertices and joints of the last step for a seeded sample of "
+                         "%d frames as DIR/vertices.npy and DIR/joints.npy (float32)" % DUMP_FRAMES)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this library's forward pass, not of --impl reference")
     args.warmup = max(args.warmup, 3)
     # rank 0 prints ONE JSON line on stdout: libraries that write to fd 1 (NCCL's version banner) go to stderr instead
     sys.stdout.flush()
@@ -354,6 +366,13 @@ def main():
     launches = int(lib.smplpp_launch_count() - launches0)
     ms_step = ms_total / args.steps
     value = world * B * P / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # taken now: the skinning leg below writes into `verts` again
+        frames = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_FRAMES), replace=False))
+        idx = torch.as_tensor(frames, device=dev)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, out in (("vertices", verts), ("joints", joints)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), out.index_select(0, idx).cpu().numpy())
 
     # the dominant kernel inside the long loop: the step minus K1
     ms_k2 = max(ms_step / P - ms_k1, 1e-6)

@@ -11,8 +11,9 @@ Writes tests/golden/ref_ik_configs.npz:
           (+-0.04) from iteration 25, and after every iteration the projection of actualPos + tangents * dphi onto
           the PRE-update mesh with the re-seated face / weights (node.cpp:949-1001; libigl is un-vendored, the
           projection is the float64 restatement oracle/smpl_oracle.py:project_points_on_mesh)
-  sb_*    shared-beta stage inputs: per-frame e and J = [theta | beta] of 16 frames (direct and VPoser) at the
-          initial state, from which the tests build the dense block-arrow system in float64
+  sb_*    shared-beta stage: inputs of 16 frames (direct and VPoser) and sb_x / sb_x_vposer, the float64 box-QP
+          solution [dtheta_1 .. dtheta_16 | dbeta] of the dense block-arrow system built from the reference's per-frame
+          e and J = [theta | beta] at the initial state (the Jacobians themselves are 1.4 MB and are not stored)
 """
 import os
 import sys
@@ -35,6 +36,55 @@ def marker_residual(e, valid):
     """mean over the valid markers of |e_m| (metres)"""
     r = np.linalg.norm(e.reshape(-1, 4)[:, :3], axis=1)
     return float(r[valid > 0].mean())
+
+
+def dense_block_arrow(J, e, theta_dim, prior=None):
+    """Dense float64 normal equations of the shared-beta problem over F frames (unknowns [x_1 .. x_F | beta]):
+    A_ff = J_f'J_f + (1e-3 + |e_f|^2) I (+ VPoser prior), A_f,beta = J_f' J_beta, A_beta,beta = sum_f J_beta'J_beta +
+    (1e-3 + sum_f |e_f|^2) I, b likewise (node/node.cpp:884-904 per frame; SURVEY 8e for the coupling)."""
+    f32 = np.float32
+    F = J.shape[0]
+    D = theta_dim
+    N = F * D + 10
+    A = np.zeros((N, N))
+    b = np.zeros(N)
+    e2_total = 0.0
+    for f in range(F):
+        Jf = J[f].astype(np.float64)
+        Af = Jf.T @ Jf
+        bf = Jf.T @ e[f]
+        e2 = float(e[f] @ e[f])
+        e2_total += e2
+        s = slice(f * D, (f + 1) * D)
+        A[s, s] = Af[:D, :D] + (np.float64(f32(1e-3)) + e2) * np.eye(D)
+        A[s, F * D:] = Af[:D, D:]
+        A[F * D:, s] = Af[D:, :D]
+        A[F * D:, F * D:] += Af[D:, D:]
+        b[s] = bf[:D]
+        b[F * D:] += bf[D:]
+        if prior is not None:
+            w, x = prior
+            A[s, s] += np.diag(w)
+            b[s] += w * x[f].astype(np.float64)
+    A[F * D:, F * D:] += (np.float64(f32(1e-3)) + e2_total) * np.eye(10)
+    return A, b
+
+
+def shared_beta_dense_solve(J, e, x_in, vposer):
+    """[dtheta_1 .. dtheta_F | dbeta] of the shared-beta step: the box QP over the dense block-arrow system, |dbeta| <= 0.5
+    (node/node.cpp:909-930), with the VPoser latent / hand prior in VPoser mode."""
+    f32 = np.float32
+    D = x_in.shape[1]
+    F = J.shape[0]
+    prior = None
+    if vposer:
+        w = np.concatenate([np.zeros(6), np.full(32, np.float64(f32(1e-5))), np.full(6, np.float64(f32(1e3)))])
+        prior = (w, x_in.astype(f32))
+    A, b = dense_block_arrow(J, e, D, prior)
+    lo = np.full(A.shape[0], -np.inf)
+    hi = np.full(A.shape[0], np.inf)
+    lo[F * D:], hi[F * D:] = -0.5, 0.5
+    return so.solve_box_qp(A, b, lo, hi)
 
 
 def assemble(vp, x):
@@ -191,8 +241,9 @@ def main():
                              optimize_beta=True, update_state=False, vposer=vp, **MOTION)
         Jv[f] = np.concatenate([r["J"][:, :44], r["J"][:, 44 + 2 * n:]], axis=1).astype(np.float32)
         ev[f] = r["e"]
-    out.update(sb_target=tgt_s, sb_valid=valid_s, sb_theta_in=xs.astype(np.float32), sb_J=Jd, sb_e=ed,
-               sb_state_in=xsv, sb_J_vposer=Jv, sb_e_vposer=ev, sb_beta_true=beta_true)
+    xs = xs.astype(np.float32)
+    out.update(sb_target=tgt_s, sb_valid=valid_s, sb_theta_in=xs, sb_x=shared_beta_dense_solve(Jd, ed, xs, False),
+               sb_state_in=xsv, sb_x_vposer=shared_beta_dense_solve(Jv, ev, xsv, True), sb_beta_true=beta_true)
     path = os.path.join(OUT, "ref_ik_configs.npz")
     np.savez_compressed(path, **out)
     print("ref_ik_configs.npz", os.path.getsize(path) // 1024, "KiB in %.0f s" % (time.time() - t_start))
