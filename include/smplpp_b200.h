@@ -250,6 +250,29 @@ int smplpp_task_positions(const smplpp_model_t * model, const smplpp_tasks_t * t
                           const float * vertices_dev, const float * vertex_weights_dev, float normal_offset,
                           float * positions_dev, float * normals_dev);
 
+/* Markers-only forward pass: SMPL::launch followed by IkTask::calcActualPos / calcActualNormal of every task
+ * (src/SMPL.cpp:671-737, src/IkTask.cpp:59-86) WITHOUT the full mesh.  Only the rest rows, posed rows and 1-ring normals
+ * of the vertices the task set depends on are computed (the face corners alone when normal_offset <= 0 and normals are
+ * not requested).
+ *   beta            (B, 10) with beta_stride >= 10, or (10) shared with beta_stride = 0
+ *   theta           (B, 25, 3): row 0 = root translation (as in smplpp_forward)
+ *   vertex_weights  (n, 3) shared with vertex_weights_stride = 0 (the MocapBody.yaml case), or (B, n, 3) with stride 3n
+ *   positions       (B, n, 3) out: calcActualPos (+ normal_offset * normal when normal_offset > 0)
+ *   normals         (B, n, 3) out, nullable: calcActualNormal
+ *   workspace       smplpp_task_forward_workspace_bytes(tasks, batch) bytes of device scratch */
+size_t smplpp_task_forward_workspace_bytes(const smplpp_tasks_t * tasks, int64_t batch);
+int smplpp_task_forward(const smplpp_model_t * model, const smplpp_tasks_t * tasks, void * stream, int64_t batch,
+                        const float * beta_dev, int64_t beta_stride, const float * theta_dev,
+                        const float * vertex_weights_dev, int64_t vertex_weights_stride, float normal_offset,
+                        float * positions_dev, float * normals_dev, void * workspace_dev, size_t workspace_bytes);
+/* The same with HOST arrays (pageable or page-locked), as a chunked pipeline: the upload of chunk c+1, the compute of
+ * chunk c and the download of chunk c-1 overlap on three internal streams; synchronises before returning.
+ * SMPLPP_TASK_CHUNK sets the frames per chunk (default 16384).  Not re-entrant per task-set handle. */
+int smplpp_task_forward_host(const smplpp_model_t * model, smplpp_tasks_t * tasks, int64_t batch,
+                             const float * beta_host, int64_t beta_stride, const float * theta_host,
+                             const float * vertex_weights_host, int64_t vertex_weights_stride, float normal_offset,
+                             float * positions_host, float * normals_host);
+
 /* Projection of the task points onto the posed mesh and the re-seated attachment (replaces the
  * igl::point_mesh_squared_distance call and the faceIdx_ / calcVertexWeights update of node/node.cpp:970-1001):
  *   vertices        (B, V, 3)   posed mesh of every frame (smplpp_forward)

@@ -745,6 +745,30 @@ public:
     check(smplpp_copy_to_host(vertexWeights.ptr(), dVw_.as<float>(), vertexWeights.data.size() * sizeof(float), nullptr));
     batch_ = b, dim_ = dim;
   }
+  /// IkTask::calcActualPos (+ calcActualNormal) of every task after SMPL::launch (src/SMPL.cpp:671-737,
+  /// src/IkTask.cpp:59-86) for B poses WITHOUT the mesh (smplpp_task_forward_host): beta (B,10) or (1,10) shared,
+  /// theta (B,25,3), vertexWeights (B,n,3) or (1,n,3) shared.  Returns the positions (B,n,3); normals (nullable) receives
+  /// the task normals (B,n,3).
+  Array calcActualPositions(const SMPL & smpl, const Array & beta, const Array & theta, const Array & vertexWeights,
+                            double normalOffset, Array * normals = nullptr)
+  {
+    const int32_t n = size();
+    if(theta.shape.size() != 3 || theta.shape[1] != JOINT_NUM + 1 || theta.shape[2] != 3)
+      throw Exception("IkTask Error: invalid IK step arguments!");
+    const int64_t b = theta.shape[0];
+    if(beta.shape.size() != 2 || beta.shape[1] != SHAPE_BASIS_DIM || (beta.shape[0] != b && beta.shape[0] != 1))
+      throw Exception("BlendShape Error: Failed to set beta!");
+    if(vertexWeights.shape.size() != 3 || vertexWeights.shape[1] != n || vertexWeights.shape[2] != 3
+       || (vertexWeights.shape[0] != b && vertexWeights.shape[0] != 1))
+      throw Exception("IkTask Error: invalid task tensors!");
+    const int64_t betaStride = (beta.shape[0] == 1 && b > 1) ? 0 : SHAPE_BASIS_DIM;
+    const int64_t vwStride = (vertexWeights.shape[0] == 1 && b > 1) ? 0 : 3 * static_cast<int64_t>(n);
+    Array pos({b, n, 3});
+    if(normals) *normals = Array({b, n, 3});
+    check(smplpp_task_forward_host(smpl.handle(), tasks_, b, beta.ptr(), betaStride, theta.ptr(), vertexWeights.ptr(),
+                                   vwStride, static_cast<float>(normalOffset), pos.ptr(), normals ? normals->ptr() : nullptr));
+    return pos;
+  }
   /// e (B, 4n): rows 4m..4m+2 = posTaskWeight (actualPos - targetPos), row 4m+3 = the normal task (node.cpp:807-820)
   Array getError() const { return detail::download(dE_.as<float>(), {batch_, 4 * size()}); }
   /// J (B, 4n, dim) in the reference's column layout [theta | phi (2n) | beta] (node.cpp:787-877)

@@ -819,6 +819,59 @@ class IkTaskSet:
                                               C.c_float(normal_offset), _ptr(pos), _ptr(nrm)))
         return (pos, nrm) if want_normals else pos
 
+    def _marker_args(self, beta, theta, vertex_weights):
+        """shapes of the markers-only forward pass -> (B, beta stride, vertex weights stride)."""
+        b = int(theta.shape[0])
+        if tuple(theta.shape) != (b, JOINT_NUM + 1, 3):
+            raise SmplppError("SMPL Error: Cannot launch a SMPL model!")
+        nb = int(np.prod(beta.shape)) // SHAPE_BASIS_DIM if beta.shape[-1] == SHAPE_BASIS_DIM else -1
+        if nb not in (1, b) or len(beta.shape) > 2:
+            raise SmplppError("BlendShape Error: Failed to set beta!")
+        nw = int(np.prod(vertex_weights.shape)) // (3 * self.n)
+        if tuple(vertex_weights.shape[-2:]) != (self.n, 3) or nw not in (1, b) or len(vertex_weights.shape) > 3:
+            raise SmplppError("IkTask Error: invalid task tensors!")
+        return b, (0 if nb == 1 and b > 1 else SHAPE_BASIS_DIM), (0 if nw == 1 and b > 1 else 3 * self.n)
+
+    def forward_positions(self, beta, theta, vertex_weights, normal_offset: float = 0.0, want_normals: bool = False):
+        """Markers-only forward pass (smplpp_task_forward): IkTask::calcActualPos (+ calcActualNormal) of every task for
+        every pose without building the mesh.  beta (B,10) or (10,) / (1,10) shared, theta (B,25,3), vertex_weights
+        (B,n,3) or (n,3) / (1,n,3) shared.  Returns positions (B,n,3) [and normals (B,n,3)] as CUDA tensors."""
+        dev = self.smpl.m__device
+        be, th, w = _dev_f32(beta, dev), _dev_f32(theta, dev), _dev_f32(vertex_weights, dev)
+        b, bstride, wstride = self._marker_args(be, th, w)
+        pos = torch.empty((b, self.n, 3), dtype=torch.float32, device=dev)
+        nrm = torch.empty((b, self.n, 3), dtype=torch.float32, device=dev) if want_normals else None
+        ws = self._workspace(lib().smplpp_task_forward_workspace_bytes(self._h, b))
+        with torch.cuda.device(dev):
+            check(lib().smplpp_task_forward(self.smpl.handle, self._h, _stream(dev), b, _ptr(be), bstride, _ptr(th),
+                                            _ptr(w), wstride, normal_offset, _ptr(pos), _ptr(nrm), _ptr(ws), ws.numel()))
+        return (pos, nrm) if want_normals else pos
+
+    def forward_positions_host(self, beta: np.ndarray, theta: np.ndarray, vertex_weights: np.ndarray,
+                               normal_offset: float = 0.0, want_normals: bool = False, out_positions=None,
+                               out_normals=None):
+        """forward_positions with HOST arrays (smplpp_task_forward_host: chunked, uploads / compute / downloads overlapped).
+        Page-locked arrays (pinned_empty) are DMA'd directly, pageable ones are staged.  Returns numpy positions (B,n,3)
+        [and normals]; out_positions / out_normals receive the result when given (C-contiguous float32 (B,n,3))."""
+        be, th, w = _np_f32(beta), _np_f32(theta), _np_f32(vertex_weights)
+        b, bstride, wstride = self._marker_args(be, th, w)
+        pos = np.empty((b, self.n, 3), np.float32) if out_positions is None else out_positions
+        nrm = None
+        if want_normals:
+            nrm = np.empty((b, self.n, 3), np.float32) if out_normals is None else out_normals
+        for a in (pos, nrm):
+            if a is not None and not (isinstance(a, np.ndarray) and a.dtype == np.float32 and a.flags["C_CONTIGUOUS"]
+                                      and a.shape == (b, self.n, 3)):
+                raise SmplppError("IkTask Error: invalid task tensors!")
+
+        def p(a):
+            return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+        with torch.cuda.device(self.smpl.m__device):
+            check(lib().smplpp_task_forward_host(self.smpl.handle, self._h, b, p(be), bstride, p(th), p(w), wstride,
+                                                 normal_offset, p(pos), p(nrm)))
+        return (pos, nrm) if want_normals else pos
+
     def assemble_theta(self, theta_state: torch.Tensor) -> torch.Tensor:
         """(B,75) -> (B,25,3) as is; (B,44) VPoser state [trans 3 | root 3 | latent 32 | hands 6] through the decoder
         (node/node.cpp:761-772)."""

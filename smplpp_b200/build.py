@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsmplpp_b200.so")
-SOURCES = ["model.cu", "forward.cu", "blend_tc.cu", "skin_tc.cu", "skin_tc3.cu", "lbs_tma.cu", "lbs_tc.cu", "host_pipe.cu", "vposer.cu", "vposer_tc.cu", "ik.cu", "ik_solve_mma.cu", "ik_poseblend_tc.cu", "ik2.cu", "ik_host.cu", "closest.cu", "sweep.cu", "io.cu"]
+SOURCES = ["model.cu", "forward.cu", "blend_tc.cu", "skin_tc.cu", "skin_tc3.cu", "lbs_tma.cu", "lbs_tc.cu", "host_pipe.cu", "vposer.cu", "vposer_tc.cu", "ik.cu", "ik_solve_mma.cu", "ik_poseblend_tc.cu", "ik2.cu", "ik_host.cu", "task_forward.cu", "closest.cu", "sweep.cu", "io.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC", "-Xcompiler", "-O3"]
 

@@ -54,7 +54,8 @@ EXPORTS = [
     "smplpp_vposer_create", "smplpp_vposer_destroy", "smplpp_vposer_decode", "smplpp_rotmat_to_axis_angle",
     "smplpp_tasks_create", "smplpp_tasks_destroy", "smplpp_tasks_count", "smplpp_tasks_vertex_count", "smplpp_tasks_rest_shape",
     "smplpp_triangle_vertex_weights", "smplpp_ik_options_default", "smplpp_ik_theta_dim", "smplpp_ik_dim",
-    "smplpp_task_positions", "smplpp_closest_points", "smplpp_sweep_grid_bounds", "smplpp_sweep_grid_winding", "smplpp_ik_workspace_bytes", "smplpp_ik_step", "smplpp_ik_jacobian", "smplpp_ik_solve_host",
+    "smplpp_task_positions", "smplpp_task_forward_workspace_bytes", "smplpp_task_forward", "smplpp_task_forward_host",
+    "smplpp_closest_points", "smplpp_sweep_grid_bounds", "smplpp_sweep_grid_winding", "smplpp_ik_workspace_bytes", "smplpp_ik_step", "smplpp_ik_jacobian", "smplpp_ik_solve_host",
     "smplpp_ik_faces_workspace_bytes", "smplpp_ik_step_faces", "smplpp_ik_reproject_workspace_bytes", "smplpp_ik_reproject",
     "smplpp_ik_shared_beta_workspace_bytes", "smplpp_ik_shared_beta_reduce", "smplpp_ik_shared_beta_apply",
     "smplpp_ik_shared_beta_step", "smplpp_task_tangents", "smplpp_solve_mocap_motion",
@@ -96,6 +97,14 @@ def lib() -> C.CDLL:
                      "smplpp_ik_reproject_workspace_bytes"):
             if hasattr(_lib, name):
                 getattr(_lib, name).restype = C.c_size_t
+        _lib.smplpp_task_forward_workspace_bytes.restype = C.c_size_t
+        _lib.smplpp_task_forward_workspace_bytes.argtypes = [C.c_void_p, C.c_int64]
+        _lib.smplpp_task_forward.argtypes = [
+            C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,
+            C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]
+        _lib.smplpp_task_forward_host.argtypes = [
+            C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_float,
+            C.c_void_p, C.c_void_p]
     return _lib
 
 

@@ -1902,6 +1902,7 @@ extern "C" void smplpp_tasks_destroy(smplpp_tasks_t * t)
 {
   if(!t) return;
   sb_release_host_solve(t);
+  sb_release_marker_pipe(t);
   for(void * ptr : t->allocations) cudaFree(ptr);
   delete t;
 }

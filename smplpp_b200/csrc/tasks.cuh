@@ -96,5 +96,26 @@ struct smplpp_tasks
     void * ws = nullptr;
     size_t ws_bytes = 0;
   } host;
+  // smplpp_task_forward_host (task_forward.cu): chunked pipeline, H2D of chunk c+1 | compute of chunk c | D2H of chunk c-1
+  struct MarkerPipe
+  {
+    cudaStream_t h2d = nullptr, compute = nullptr, d2h = nullptr;
+    cudaEvent_t uploaded[2] = {nullptr, nullptr}; // inputs of the chunk on the device (h2d stream)
+    cudaEvent_t computed[2] = {nullptr, nullptr}; // outputs of the chunk written, inputs consumed (compute stream)
+    cudaEvent_t drained[2] = {nullptr, nullptr};  // outputs of the chunk copied out (d2h stream)
+    void * dev_in[2] = {nullptr, nullptr};        // theta | beta (per frame) | vertex weights (per frame) of one chunk
+    size_t dev_in_bytes = 0;
+    void * dev_out[2] = {nullptr, nullptr};       // positions | normals of one chunk
+    size_t dev_out_bytes = 0;
+    void * dev_shared = nullptr;                  // shared beta | shared vertex weights
+    size_t dev_shared_bytes = 0;
+    void * ws = nullptr;                          // smplpp_task_forward workspace of one chunk
+    size_t ws_bytes = 0;
+    void * pin_in[2] = {nullptr, nullptr};        // staging of pageable inputs
+    size_t pin_in_bytes = 0;
+    void * pin_out[2] = {nullptr, nullptr};       // staging of pageable outputs
+    size_t pin_out_bytes = 0;
+  } marker;
 };
 void sb_release_host_solve(smplpp_tasks * t);
+void sb_release_marker_pipe(smplpp_tasks * t);
