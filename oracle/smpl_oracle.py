@@ -161,6 +161,11 @@ class SmplModel:
         return SmplModel(faces, _t(p.shape_blend_shapes), _t(p.pose_blend_shapes), _t(p.vertices_template),
                          _t(p.joint_regressor), parents, _t(p.weights), adj)
 
+    def to(self, dtype: torch.dtype) -> "SmplModel":
+        """A copy with the floating-point tensors in `dtype` (face indices, parents and adjacency shared)."""
+        return SmplModel(self.face_indices, self.shape_basis.to(dtype), self.pose_basis.to(dtype), self.templ.to(dtype),
+                         self.joint_regressor.to(dtype), self.parents, self.weights.to(dtype), self.adjacent)
+
 
 @dataclass
 class ForwardResult:
@@ -352,6 +357,10 @@ class VPoserDecoder:
         return VPoserDecoder(*[_t(p[k]) for k in ("decoder_net.0.weight", "decoder_net.0.bias", "decoder_net.3.weight",
                                                   "decoder_net.3.bias", "decoder_net.5.weight", "decoder_net.5.bias")])
 
+    def to(self, dtype: torch.dtype) -> "VPoserDecoder":
+        """A copy with the weights in `dtype`."""
+        return VPoserDecoder(*[w.to(dtype) for w in (self.w0, self.b0, self.w3, self.b3, self.w5, self.b5)])
+
     def mlp(self, z):
         lrelu = torch.nn.functional.leaky_relu
         h = lrelu(torch.nn.functional.linear(z, self.w0, self.b0), 0.01)
@@ -422,8 +431,8 @@ class IkResult:
     A: np.ndarray
     b: np.ndarray
     delta: np.ndarray
-    theta_state: np.ndarray  # updated g_theta (float32)
-    beta: np.ndarray  # updated g_beta (float32)
+    theta_state: np.ndarray  # updated g_theta (in the dtype of the call)
+    beta: np.ndarray  # updated g_beta (in the dtype of the call)
     vertex_weights: np.ndarray  # (n,3) after the re-weighting of node.cpp:803-804
     actual_pos: np.ndarray  # (n,3) marker positions (pre-update mesh, with the normal offset)
     skipped: bool
@@ -442,12 +451,34 @@ def assemble_theta(g_theta: torch.Tensor, vposer: Optional[VPoserDecoder]) -> to
 
 def ik_iteration(model: SmplModel, tasks: List[IkTask], theta_state: np.ndarray, beta: np.ndarray,
                  vposer: Optional[VPoserDecoder] = None, optimize_beta: bool = False, enable_qp: bool = True,
-                 skip_if_too_few: bool = False) -> IkResult:
+                 skip_if_too_few: bool = False, dtype: torch.dtype = torch.float32) -> IkResult:
     """One pass of node/node.cpp:705-968 for ONE frame.  `tasks` carry targets/weights/limits and are
-    updated in place (vertex_weights, tangents) as the node does."""
+    updated in place (vertex_weights, tangents) as the node does.
+
+    dtype=torch.float32 is the reference's arithmetic.  dtype=torch.float64 runs the same operations in double precision
+    (a reference for the reference, where float32 autograd is ill-conditioned): the model and the VPoser decoder must then
+    be float64 copies (SmplModel.to / VPoserDecoder.to), the tensors of `tasks` are cast to float64 in place, and the
+    torch default dtype is float64 for the duration of the call (the restated reference builds constants with
+    torch.zeros / torch.eye) and restored afterwards, also when the call raises."""
+    if model.templ.dtype != dtype or (vposer is not None and vposer.w0.dtype != dtype):
+        raise TypeError("ik_iteration(dtype=%s) needs the model and the decoder in that dtype (use .to(dtype))" % dtype)
+    prev = torch.get_default_dtype()
+    torch.set_default_dtype(dtype)
+    try:
+        if dtype != torch.float32:
+            for t in tasks:
+                for k in ("target_pos", "target_normal", "vertex_weights", "tangents", "phi"):
+                    setattr(t, k, getattr(t, k).to(dtype))
+        return _ik_iteration(model, tasks, theta_state, beta, vposer, optimize_beta, enable_qp, skip_if_too_few, dtype)
+    finally:
+        torch.set_default_dtype(prev)
+
+
+def _ik_iteration(model, tasks, theta_state, beta, vposer, optimize_beta, enable_qp, skip_if_too_few, dtype):
     n = len(tasks)
-    g_theta = torch.tensor(np.asarray(theta_state, dtype=np.float32).reshape(-1), requires_grad=True)
-    g_beta = torch.tensor(np.asarray(beta, dtype=np.float32).reshape(-1), requires_grad=bool(optimize_beta))
+    np_dtype = np.float32 if dtype == torch.float32 else np.float64
+    g_theta = torch.tensor(np.asarray(theta_state, dtype=np_dtype).reshape(-1), requires_grad=True)
+    g_beta = torch.tensor(np.asarray(beta, dtype=np_dtype).reshape(-1), requires_grad=bool(optimize_beta))
     theta_dim = g_theta.numel()
     assert theta_dim == (LATENT_DIM + 12 if vposer is not None else 3 * (JOINT_NUM + 1))
     phi_dim, beta_dim = 2 * n, (SHAPE_DIM if optimize_beta else 0)
@@ -519,9 +550,9 @@ def ik_iteration(model: SmplModel, tasks: List[IkTask], theta_state: np.ndarray,
     new_theta = g_theta.detach().numpy().copy()
     new_beta = g_beta.detach().numpy().copy()
     if not skipped:  # :946-968
-        new_theta = new_theta + delta[:theta_dim].astype(np.float32)
+        new_theta = new_theta + delta[:theta_dim].astype(np_dtype)
         if optimize_beta:
-            new_beta = new_beta + delta[theta_dim + phi_dim:].astype(np.float32)
+            new_beta = new_beta + delta[theta_dim + phi_dim:].astype(np_dtype)
     for t in tasks:
         t.phi = t.phi.detach()
         t.vertex_weights = t.vertex_weights.detach()
