@@ -114,13 +114,9 @@ int smplpp_host_unregister(void * ptr);
 
 /* TEST / TUNING switch, process-wide (atomic; it affects the calls issued after it, on every handle): production code
  * never needs it - every default is "auto".  The parity tests use it to run one input through every implementation.
- *   0..6      smplpp_forward: 0 = auto, 1 = FFMA fused blend+skinning, 2 = tcgen05 3xTF32 fused blend+skinning,
- *             3 = unfused (blend GEMM -> rest shape -> standalone skinning), 4 = tcgen05 3xBF16 fused blend+skinning
- *             (faster, ~1.5e-6 m contraction error instead of ~3e-8 m), 5 = tcgen05 3xFP16 blend + skinning matrices on the
- *             tensor cores (one CTA per tile), 6 = the persistent pipelined form of 5 (the default when available).
- *             Variants 2 and 4 need an even vertex count >= 128 and <= 4 skinning influences per vertex; 5 / 6 an even
- *             vertex count >= 128 only.
- *   100 / 101 grid order of the variant-2/4 kernel
+ *   0 1 3 6   smplpp_forward: 0 = auto, 1 = FFMA fused blend+skinning, 3 = unfused (blend GEMM -> rest shape ->
+ *             standalone skinning), 6 = tcgen05 3xFP16 blend + skinning matrices on the tensor cores, persistent and
+ *             pipelined (the default when available: a CC 10.x device and an even vertex count >= 128).
  *   200..202  standalone skinning: FFMA TMA pipeline / FFMA register kernel / tcgen05 (default)
  *   300 / 301 VPoser decoder Jacobian: tcgen05 (default) / FFMA
  *   400..402  IK step: auto (two kernels for shared attachments, fused kernel for per-frame ones) / two kernels / fused

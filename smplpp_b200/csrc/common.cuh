@@ -103,20 +103,11 @@ struct ModelDev
   // originals kept for the task builder and the generic module kernels
   float * weights_dense = nullptr; // (V, 24)
   uint32_t * vert_jmask = nullptr; // (V) joints whose rotation moves the vertex (ancestor closure of its influences)
-  // tcgen05 blend variant (blend_tc.cu): split basis [part hi|lo][tile][plane x|y|z][128][224] as bf16 ([0]) and
-  // tf32-rounded fp32 ([1]) with their TMA tensor maps (CUtensorMap is 128 bytes, 64-byte aligned)
-  void * basis_split[2] = {nullptr, nullptr};
-  alignas(64) unsigned char tmapA[2][128] = {};
-  int tc_tiles = 0;
-  bool tc_ready = false;
-  // tcgen05 blend + tensor-core skinning (skin_tc.cu): fp16 hi | lo split basis scaled by 2^tc2_basis_exp
-  void * basis_f16 = nullptr;
-  alignas(64) unsigned char tmapA16[128] = {};
-  int tc2_basis_exp = 0;
-  int tc2_tiles = 0;
-  bool tc2_ready = false;
-  // persistent pipelined variant (skin_tc3.cu): shares the tc2 model data
+  // tcgen05 blend + skinning (skin_tc3.cu): fp16 hi | lo split basis scaled by 2^tc3_basis_exp.  tc3_ready also
+  // gates the tcgen05 standalone skinning kernel (lbs_tc.cu).
   void * basis_img16 = nullptr; // [tile][K-block][hi | lo][plane][128][32 fp16]: SWIZZLE_64B stage images
+  int tc3_basis_exp = 0;
+  int tc3_tiles = 0;
   bool tc3_ready = false;
   int sm_count = 0;
 };

@@ -924,12 +924,6 @@ int launch_lbs(const ModelDev & d, cudaStream_t st, int B, const float * rest, c
 
 extern "C" int smplpp_set_forward_variant(int variant)
 {
-  // 100 / 101: tuning switch for the grid order of the tcgen05 kernel (tile-fastest / frames-fastest)
-  if(variant == 100 || variant == 101)
-  {
-    g_tc_grid_order = variant - 100;
-    return SMPLPP_OK;
-  }
   // 200 / 201 / 202: standalone skinning kernel (FFMA per-warp TMA pipelines / FFMA register-pipelined kernel / skinning
   // matrices on tcgen05, the default; the FFMA kernels are bound by FFMA issue at ~3.2 TB/s, see DESIGN.md §4)
   if(variant == 300 || variant == 301) // VPoser Jacobian: 300 tensor cores (default), 301 FFMA kernel
@@ -962,7 +956,8 @@ extern "C" int smplpp_set_forward_variant(int variant)
     g_poseblend_variant = variant - 420;
     return SMPLPP_OK;
   }
-  if(variant < 0 || variant > 6) return fail(SMPLPP_ERR_INVALID, "SMPL", "unknown forward variant");
+  if(variant != 0 && variant != 1 && variant != 3 && variant != 6)
+    return fail(SMPLPP_ERR_INVALID, "SMPL", "unknown forward variant");
   g_forward_variant = variant;
   return SMPLPP_OK;
 }
@@ -974,8 +969,7 @@ extern "C" size_t smplpp_forward_workspace_bytes(const smplpp_model_t * model, i
   size_t bytes = 512;
   bytes += align_up(bpad * kBlendK * sizeof(float));         // coefficients (A operand)
   bytes += align_up(bpad * kJoints * 12 * sizeof(float));    // relative transforms 3x4
-  bytes += tc_coef_split_bytes(batch);                      // hi / lo coefficient parts (tcgen05 variants)
-  bytes += std::max(tc2_frame_operand_bytes(batch), tc3_frame_operand_bytes(batch));                  // fp16 hi / lo coefficients + transforms (variant 5)
+  bytes += tc3_frame_operand_bytes(batch);                  // fp16 hi / lo coefficient + transform stage images (variant 6)
   bytes += align_up(static_cast<size_t>(batch) * model->d.V * 3 * sizeof(float)); // rest shape (unfused variant)
   return bytes;
 }
@@ -997,23 +991,20 @@ extern "C" int smplpp_forward(const smplpp_model_t * model, void * stream, int64
   ws += align_up(bpad * kBlendK * sizeof(float));
   float * xforms = reinterpret_cast<float *>(ws);
   ws += align_up(bpad * kJoints * 12 * sizeof(float));
-  void * coef_split = ws;
-  ws += tc_coef_split_bytes(batch);
-  void * tc2_scratch = ws;
-  ws += std::max(tc2_frame_operand_bytes(batch), tc3_frame_operand_bytes(batch));
+  void * tc3_scratch = ws;
+  ws += tc3_frame_operand_bytes(batch);
   float * rest_ws = reinterpret_cast<float *>(ws);
 
   const bool need_verts = vertices != nullptr;
   const bool need_rest = rest_shape != nullptr;
   int variant = g_forward_variant;
-  if(variant == 0) variant = model->d.tc3_ready ? 6 : (model->d.tc2_ready ? 5 : (model->d.tc_ready ? 2 : 1));
-  if(((variant == 2 || variant == 4) && !model->d.tc_ready) || (variant == 5 && !model->d.tc2_ready)
-     || (variant == 6 && !model->d.tc3_ready))
+  if(variant == 0) variant = model->d.tc3_ready ? 6 : 1;
+  if(variant == 6 && !model->d.tc3_ready)
     return fail(SMPLPP_ERR_INVALID, "SMPL", "tcgen05 blend variant is not available for this model");
   // K1 writes the stage images of K2''' itself when that kernel follows
   const bool fused_images = variant == 6 && need_verts && !need_rest;
   int rc = launch_pose_chain(d, st, B, beta, beta_stride, theta, (need_verts || need_rest) ? coef : nullptr, xforms,
-                             joints, transforms, fused_images ? tc2_scratch : nullptr);
+                             joints, transforms, fused_images ? tc3_scratch : nullptr);
   if(rc != SMPLPP_OK) return rc;
   if(need_rest || (need_verts && variant == 3))
   {
@@ -1026,11 +1017,7 @@ extern "C" int smplpp_forward(const smplpp_model_t * model, void * stream, int64
   if(need_verts)
   {
     if(variant == 6)
-      rc = launch_blend_skin_tc3(d, st, B, coef, xforms, tc2_scratch, theta, vertices, /*images_ready=*/true);
-    else if(variant == 5)
-      rc = launch_blend_skin_tc2(d, st, B, coef, xforms, tc2_scratch, theta, vertices);
-    else if(variant == 2 || variant == 4)
-      rc = launch_blend_skin_tc(d, st, B, coef, coef_split, xforms, theta, vertices, variant == 2);
+      rc = launch_blend_skin_tc3(d, st, B, coef, xforms, tc3_scratch, theta, vertices, /*images_ready=*/true);
     else
       rc = launch_blend_skin_ffma(d, st, B, coef, xforms, theta, vertices, true);
   }

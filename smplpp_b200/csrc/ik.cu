@@ -1851,10 +1851,9 @@ extern "C" int smplpp_tasks_create(const smplpp_model_t * model, int32_t n, cons
   // none of them may be reachable through the compact view (lbs_tc_usable() would otherwise accept an even nU >= 128
   // and skin sub-vertex u with the weights of model vertex u)
   t->sub.weights_dense = nullptr;
-  t->sub.basis_split[0] = t->sub.basis_split[1] = nullptr;
-  t->sub.basis_f16 = nullptr, t->sub.basis_img16 = nullptr;
-  t->sub.tc_ready = t->sub.tc2_ready = t->sub.tc3_ready = false;
-  t->sub.tc_tiles = t->sub.tc2_tiles = 0;
+  t->sub.basis_img16 = nullptr;
+  t->sub.tc3_ready = false;
+  t->sub.tc3_tiles = 0;
   t->sub.faces = nullptr, t->sub.adj_offset = nullptr, t->sub.adj_faces = nullptr;
   t->sub_corner = t->sub;
   t->sub_corner.V = nCorner;

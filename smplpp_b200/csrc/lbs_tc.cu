@@ -6,8 +6,8 @@
 // The FFMA kernels (lbs_kernel, lbs_tma_kernel) spend ~44 FMAs per vertex and frame on forming
 // sum_j W[v,j] G'_j and are bound by FFMA issue at ~3.2 TB/s.  Here M[v,f] = sum_j W[v,j] G'[f,j] is a GEMM on the
 // tensor cores (128 vertices x (8 frames x 12), K = 24 -> 32, fp16 hi | lo split, three products, fp32 accumulate in
-// TMEM; same operand formats as skin_tc.cu) and the CUDA cores only apply M to the rest position: 12 FMAs per
-// vertex and frame.
+// TMEM; same operand split as skin_tc3.cu, skin_common.cuh) and the CUDA cores only apply M to the rest position:
+// 12 FMAs per vertex and frame.
 //
 // CTA = 128 vertices x a chunk of frames, walked in 8-frame sub-batches:
 //   warps 0, 18-20 producers (producer i owns sub-batches i, i+4, ...; lane t issues frame t's copy): per sub-batch one ring slot = the transforms (TMA tensor load, fp16 hi | lo, K-major) + the
@@ -340,11 +340,8 @@ __global__ void __launch_bounds__(k3c::THREADS, 1) lbs_tc_kernel(const __grid_co
   if(warp == 1) ptx::tmem_dealloc<TMEM_COLS>(tmem_base);
 }
 
-namespace
+namespace sb
 {
-using EncodeTiledFn = CUresult (*)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 EncodeTiledFn encode_fn()
 {
   static EncodeTiledFn fn = nullptr;
@@ -360,13 +357,10 @@ EncodeTiledFn encode_fn()
   });
   return fn;
 }
-} // namespace
 
-namespace sb
-{
 bool lbs_tc_usable(const ModelDev & d, const float * rest, const float * out, const float * xforms)
 {
-  return d.tc2_ready && (d.V & 1) == 0 && d.V >= k3c::MV && (reinterpret_cast<uintptr_t>(rest) & 15) == 0
+  return d.tc3_ready && (d.V & 1) == 0 && d.V >= k3c::MV && (reinterpret_cast<uintptr_t>(rest) & 15) == 0
          && (reinterpret_cast<uintptr_t>(out) & 7) == 0 && (reinterpret_cast<uintptr_t>(xforms) & 15) == 0 && rest != out
          && encode_fn() != nullptr;
 }

@@ -13,8 +13,6 @@
 // A frame is V * 12 bytes = 82 680 B for SMPL, i.e. 8 mod 16: every other frame starts 8 bytes off a 16-byte
 // boundary.  Loads copy the enclosing aligned range (data lands at stage + lo, lo in {0, 8}); stores send the
 // aligned interior with the bulk copy and the 8-byte head / tail with ordinary stores.
-#include <cstdlib>
-
 #include "forward.cuh"
 #include "tc_ptx.cuh"
 
@@ -110,7 +108,7 @@ __global__ void __launch_bounds__(k3t::THREADS, 2)
                    const float * __restrict__ lbs_wsum, const int8_t * __restrict__ group_nj,
                    const uint8_t * __restrict__ group_joint, const float * __restrict__ group_w, int V, int Vpad, int kmax,
                    int B, const float * __restrict__ rest, const float * __restrict__ xforms, const float * __restrict__ root,
-                   int root_stride, float * __restrict__ out, int dbg_copy_only)
+                   int root_stride, float * __restrict__ out)
 {
   using namespace k3t;
   using L = Layout<FRC, S>;
@@ -226,7 +224,7 @@ __global__ void __launch_bounds__(k3t::THREADS, 2)
     const uint32_t my = st_addr + lo + 48u * lane;
     const uint32_t gf = gs_addr + static_cast<uint32_t>(f) * (kJoints * kXformFloats * 4);
     const float tx = Tr[4 * f], ty = Tr[4 * f + 1], tz = Tr[4 * f + 2];
-    if(!dbg_copy_only) switch(nj_max)
+    switch(nj_max)
     {
       case 0:
       case 1: skin_in_place<1>(my, lo, gf, joff, gw, iw, tx, ty, tz); break;
@@ -306,31 +304,12 @@ int launch_lbs_tma(const ModelDev & d, cudaStream_t st, int B, const float * res
                    int root_stride, float * out)
 {
   const int slices = (d.V + k3t::SLICE - 1) / k3t::SLICE;
-  static int cfg = -1, copy_only = 0;
-  if(cfg < 0)
-  {
-    cfg = getenv("SMPLPP_LBS_CFG") ? atoi(getenv("SMPLPP_LBS_CFG")) : 0;
-    copy_only = getenv("SMPLPP_LBS_COPY") ? 1 : 0;
-  }
-#define SB_LBS_TMA(FRC, S)                                                                                             \
-  {                                                                                                                    \
-    using L = k3t::Layout<FRC, S>;                                                                                     \
-    SB_CUDA(cudaFuncSetAttribute(lbs_tma_kernel<FRC, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::BYTES));      \
-    dim3 grid((slices + k3t::WARPS - 1) / k3t::WARPS, (B + FRC - 1) / FRC);                                            \
-    lbs_tma_kernel<FRC, S><<<grid, k3t::THREADS, L::BYTES, st>>>(d.lbs_joint, d.lbs_weight, d.lbs_wsum, d.group_nj,    \
-                                                                  d.group_joint, d.group_w, d.V, d.Vpad, d.kmax, B,    \
-                                                                  rest, xforms, root, root_stride, out, copy_only);    \
-  }
-  switch(cfg)
-  {
-    case 1: SB_LBS_TMA(16, 6) break;
-    case 2: SB_LBS_TMA(32, 4) break;
-    case 3: SB_LBS_TMA(8, 4) break;
-    case 4: SB_LBS_TMA(16, 2) break;
-    case 5: SB_LBS_TMA(32, 8) break;
-    default: SB_LBS_TMA(16, 4) break;
-  }
-#undef SB_LBS_TMA
+  using L = k3t::Layout<kFrc, kStages>;
+  SB_CUDA(cudaFuncSetAttribute(lbs_tma_kernel<kFrc, kStages>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::BYTES));
+  dim3 grid((slices + k3t::WARPS - 1) / k3t::WARPS, (B + kFrc - 1) / kFrc);
+  lbs_tma_kernel<kFrc, kStages><<<grid, k3t::THREADS, L::BYTES, st>>>(d.lbs_joint, d.lbs_weight, d.lbs_wsum, d.group_nj,
+                                                                      d.group_joint, d.group_w, d.V, d.Vpad, d.kmax, B,
+                                                                      rest, xforms, root, root_stride, out);
   SB_LAUNCHED();
   return SMPLPP_OK;
 }

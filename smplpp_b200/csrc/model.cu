@@ -242,13 +242,11 @@ extern "C" int smplpp_model_create(const smplpp_model_desc * desc, smplpp_model_
   if(upload(&d.adj_offset, m->h_adj_offset) != SMPLPP_OK) return SMPLPP_ERR_CUDA;
   if(upload(&d.adj_faces, m->h_adj_faces) != SMPLPP_OK) return SMPLPP_ERR_CUDA;
 
-  if(tc_prepare_model(d) != SMPLPP_OK) return SMPLPP_ERR_CUDA;
   {
     float mx = 0.f; // largest pose / shape basis entry (the template column stays out of the tensor-core product)
     for(size_t r = 0; r < static_cast<size_t>(3) * V; r++)
       for(int k = 0; k < kPoseDim + kShapeDim; k++) mx = std::max(mx, std::fabs(m->h_basis[r * kBlendK + k]));
-    if(tc2_prepare_model(d, mx) != SMPLPP_OK) return SMPLPP_ERR_CUDA;
-    if(tc3_prepare_model(d) != SMPLPP_OK) return SMPLPP_ERR_CUDA;
+    if(tc3_prepare_model(d, mx) != SMPLPP_OK) return SMPLPP_ERR_CUDA;
   }
   *out = guard.release();
   return SMPLPP_OK;
@@ -272,9 +270,7 @@ extern "C" void smplpp_model_destroy(smplpp_model_t * m)
   cudaFree(d.adj_faces);
   cudaFree(d.weights_dense);
   cudaFree(d.vert_jmask);
-  tc_release_model(d);
   tc3_release_model(d);
-  tc2_release_model(d);
   release_host_pipe(m);
   delete m;
 }

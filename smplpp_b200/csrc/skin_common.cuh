@@ -1,5 +1,5 @@
 // Pieces shared by the two kernels that compute the skinning matrices M[v,f] = sum_j W[v,j] G'[f,j] on tcgen05
-// (skin_tc.cu: fused with the blend contraction; lbs_tc.cu: standalone skinning): the fp16 hi | lo operand formats.
+// (skin_tc3.cu: fused with the blend contraction; lbs_tc.cu: standalone skinning): the fp16 hi | lo operand formats.
 #pragma once
 #include <cuda_fp16.h>
 

@@ -8,8 +8,7 @@
 //   M[v,f]      = sum_j W[v,j] G'[f,j]  (3x4 per vertex and frame)  GEMM 2: 128 vertices x (8 frames x 12), K = 24 -> 32
 //   vert[v,f]   = M[v,f] [rest; 1] / sum_j W[v,j] + trans[f]        epilogue: 12 FMA per vertex and frame
 //
-// What changed against K2'' (skin_tc.cu), whose CTA ran wait(3.2 k) -> GEMM 1 (8.6 k) -> GEMM 2 + epilogue (11 k cycles)
-// back to back with the tensor pipe idle for two thirds of the time:
+// Work and pipeline (DESIGN.md 4.1 has the measurements):
 //   * one persistent CTA per SM walks a contiguous range of (vertex tile, frame block) work items;
 //   * when GEMM 1 of an item completes, the sixteen epilogue warps DRAIN its 288 accumulator columns into registers
 //     (72 per thread, pre-scaled by 1 / sum_j W), which frees the TMEM columns: one thread then issues the 126 MMAs of
@@ -20,8 +19,10 @@
 //     warp owns are 24 adjacent accumulator columns (6 tcgen05.ld per drain instead of 36).
 //   * every operand tile is stored in global memory as the exact (SWIZZLE_64B) shared-memory image of its pipeline
 //     stage, so a stage is two contiguous cp.async.bulk copies (48 KB basis + 12 KB coefficients) and a transform
-//     sub-batch is one (12 KB): no tensor maps, a handful of large copies per item (DESIGN.md 4.1 has the measurements).
-// Precision is that of K2'': fp16 hi + lo split of every operand, hi.hi + lo.hi + hi.lo in fp32 TMEM.
+//     sub-batch is one (12 KB): no tensor maps, a handful of large copies per item.
+// Precision: both GEMMs are fp32 in the reference.  Every operand is split into fp16 hi + lo (power-of-two pre-scaled
+// so that lo stays a normal fp16) and three products are accumulated in fp32 TMEM, hi.hi + lo.hi + hi.lo (~2^-22
+// relative).  The ~1 m template stays out of GEMM 1 and is added in fp32.
 //
 // TMEM (512 columns): [0,288) rest accumulators (x | y | z planes x 96 frames), [288,480) two 96-column buffers of
 // skinning matrices (8 frames x 12), [480,512) the W tile (A operand of GEMM 2, fp16 hi | lo).
@@ -30,10 +31,6 @@
 // 112 registers each (four per TMEM lane quadrant, one per frame pair of an 8-frame sub-batch).
 #include <cuda.h>
 #include <cuda_fp16.h>
-
-#include <cstdio>
-#include <cstdlib>
-#include <vector>
 
 #include "forward.cuh"
 #include "skin_common.cuh"
@@ -56,8 +53,6 @@ struct Params
   const float * wsum;           // (Vpad)
   const float * theta;          // (B, 25, 3): row 0 = root translation
   float * out;                  // (B, V, 3)
-  long long * dbg;              // optional per-CTA timestamps (SMPLPP_TC3_DBG)
-  int dbg_mode;                 // DBG build only (SMPLPP_TC3_DBG = bit mask): 1 no matrix tcgen05.ld, 2 no stores, 4 no GEMM 2 MMAs, 8 no GEMM 1 MMAs, 16 no drain loads, 32 no stage ring, 64 no transform ring, 128 no epilogue arithmetic, 256 no matrix-buffer hand-off, 512 no drain hand-off (results are wrong: timing decomposition)
 };
 
 } // namespace tc3
@@ -135,13 +130,13 @@ __global__ void frame_images3_kernel(const float * __restrict__ coef, const floa
   }
 }
 
-template<int STAGES, int GSLOTS, int EPI, bool DBG = false>
+template<int STAGES, int GSLOTS>
 __global__ void __launch_bounds__(tc3::THREADS, 1)
     blend_skin_tc3_kernel(const tc3::Params p)
 {
   using namespace tc3;
-  using L = Layout<STAGES, GSLOTS, EPI>;
-  constexpr int OFF_G = L::OFF_G, OFF_STG = L::OFF_STG, OFF_BAR = L::OFF_BAR;
+  using L = Layout<STAGES, GSLOTS>;
+  constexpr int OFF_G = L::OFF_G, OFF_BAR = L::OFF_BAR;
   extern __shared__ uint8_t smem_raw[];
   uint8_t * smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t * bars = reinterpret_cast<uint64_t *>(smem + OFF_BAR);
@@ -194,11 +189,6 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
   __syncthreads();
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  long long * dbg = (DBG && p.dbg) ? p.dbg + static_cast<size_t>(blockIdx.x) * 256 : nullptr;
-  // DBG build: cycles the MMA thread / one epilogue warp spend blocked in each kind of wait (SMPLPP_TC3_DBG)
-  long long w_stage = 0, w_gfull = 0, w_mempty = 0, w_rest = 0, w_pfull = 0, w_mfull = 0;
-#define TC3_OFF(bit) (DBG && (p.dbg_mode & (bit)))
-#define TC3_TIMED(acc, stmt) do { if constexpr(DBG) { const long long t_ = clock64(); stmt; acc += clock64() - t_; } else { stmt; } } while(0)
 
   if(warp < CTRL_WARPS)
   {
@@ -211,7 +201,7 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
     // producer thread with plain blocking waits.  A single polling producer over both rings performed the same.)
     if(ptx::elect_one())
     {
-      const int total_kb = TC3_OFF(32) ? 0 : nit * NKB;
+      const int total_kb = nit * NKB;
       // (An L2 prefetch of all seven K-blocks of the first item at kernel start was measured: no gain.)
       // The reload of a stage is on the critical path of the GEMM 1 issuer (a quarter of its samples are stage waits):
       // source addresses (two integer divisions) are ready BEFORE the wait, barriers and stages are 32-bit shared addresses.
@@ -226,7 +216,6 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
         ptx::mbar_expect_tx_a(fbar, STAGE);
         ptx::bulk_load_1d_a(dst, srca, 2 * A_PART, fbar);
         ptx::bulk_load_1d_a(dst + 2 * A_PART, srcb, 2 * B_PART, fbar);
-        if(dbg && kbn < 14) dbg[34 + kbn] = clock64();
         if(++kb == NKB)
         {
           kb = 0;
@@ -240,7 +229,7 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
     // ---- producer of the transform sub-batch ring ----
     if(ptx::elect_one())
     {
-      const int total_g = TC3_OFF(64) ? 0 : nit * NSUB;
+      const int total_g = nit * NSUB;
       int sb = 0, fb = it0 % p.nfb;
       for(int gn = 0; gn < total_g; gn++)
       {
@@ -304,42 +293,36 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
         const uint32_t st16 = smem16 + s * (STAGE >> 4);
         if((h & 1) == 0)
         {
-          if(!TC3_OFF(32)) TC3_TIMED(w_stage, ptx::mbar_wait_a(a_full + 8 * s, (kbn / STAGES) & 1));
+          ptx::mbar_wait_a(a_full + 8 * s, (kbn / STAGES) & 1);
           ptx::tc_fence_after();
-          if(dbg && kbn < 14) dbg[48 + kbn] = clock64();
 #pragma unroll
-          for(int i = 0; i < 9; i++)
-            if(!DBG || !(p.dbg_mode & 8)) g1_mma(st16, 0, i, (h == 0 && i < 3) ? 0u : 1u);
+          for(int i = 0; i < 9; i++) g1_mma(st16, 0, i, (h == 0 && i < 3) ? 0u : 1u);
         }
         else
         {
 #pragma unroll
-          for(int i = 0; i < 9; i++)
-            if(!DBG || !(p.dbg_mode & 8)) g1_mma(st16, 1, i, 1u);
-          if(!TC3_OFF(32)) ptx::tc_commit_a(a_empty + 8 * s);
+          for(int i = 0; i < 9; i++) g1_mma(st16, 1, i, 1u);
+          ptx::tc_commit_a(a_empty + 8 * s);
         }
       };
-      if(dbg) dbg[0] = clock64();
       if(nit > 0 && warp == 3)
       {
 #pragma unroll
         for(int h = 0; h < 2 * NKB; h++) g1_half(h, 0);
-        if(!TC3_OFF(512)) ptx::tc_commit_a(a_pfull);
+        ptx::tc_commit_a(a_pfull);
       }
-      if(dbg) dbg[1] = clock64();
       if(warp == 3)
       {
         // ---- GEMM 1 issuer: the 126 MMAs of item k + 1 as soon as item k's accumulators have been drained into the epilogue
         //      warps' registers; the stage ring and the tensor queue pace it ----
         for(int k = 0; k + 1 < nit; k++)
         {
-          if(!TC3_OFF(512)) TC3_TIMED(w_rest, ptx::mbar_wait_a(a_rest, k & 1));
+          ptx::mbar_wait_a(a_rest, k & 1);
           ptx::tc_fence_after();
 #pragma unroll
           for(int h = 0; h < 2 * NKB; h++) g1_half(h, (k + 1) * NKB);
-          if(!TC3_OFF(512)) ptx::tc_commit_a(a_pfull);
+          ptx::tc_commit_a(a_pfull);
         }
-        if(dbg) dbg[64] = w_stage, dbg[67] = w_rest, dbg[69] = clock64();
       }
       // ---- GEMM 2 issuer (warp 1): the twelve sub-batches of every item, two matrix buffers ----
       int wcount = 0, prev_tile = -1;
@@ -358,20 +341,17 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
         for(int sb = 0; sb < NSUB; sb++)
         {
           const int b = sb & 1, gs = sb % GSLOTS;
-          if(!TC3_OFF(64)) TC3_TIMED(w_gfull, ptx::mbar_wait_a(a_gfull + 8 * gs, (sb / GSLOTS) & 1));
-          if(!TC3_OFF(256)) TC3_TIMED(w_mempty, ptx::mbar_wait_a(a_mempty + 8 * b, ((sb >> 1) & 1) ^ 1));
+          ptx::mbar_wait_a(a_gfull + 8 * gs, (sb / GSLOTS) & 1);
+          ptx::mbar_wait_a(a_mempty + 8 * b, ((sb >> 1) & 1) ^ 1);
           ptx::tc_fence_after();
           const uint32_t sg16 = smem16 + ((OFF_G + gs * G_STAGE) >> 4);
           const uint32_t dm = tmem_base + COL_M + b * SUBN;
 #pragma unroll
-          for(int j = 0; j < 6; j++)
-            if(!DBG || !(p.dbg_mode & 4)) g2_mma(dm, aw, sg16, j);
-          if(!TC3_OFF(256)) ptx::tc_commit_a(a_mfull + 8 * b);
-          if(!TC3_OFF(64)) ptx::tc_commit_a(a_gempty + 8 * gs);
+          for(int j = 0; j < 6; j++) g2_mma(dm, aw, sg16, j);
+          ptx::tc_commit_a(a_mfull + 8 * b);
+          ptx::tc_commit_a(a_gempty + 8 * gs);
         }
-        if(dbg && k < 30) dbg[2 + k] = clock64();
       }
-      if(dbg && warp == 1) dbg[65] = w_gfull, dbg[66] = w_mempty, dbg[68] = clock64();
     }
   }
   }
@@ -382,7 +362,6 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
     const int q = warp & 3;        // TMEM lane quadrant this warp may access (hardware rule: warp id % 4)
     const int fp = ew >> 2;        // which frame pair of every 8-frame sub-batch
     const uint32_t lane_taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-    const uint32_t my_stg = ptx::smem_u32(smem + OFF_STG) + ew * STG_FLOATS * 4;
     const float sp = p.scale_p;
     // barriers as 32-bit shared addresses, frame stride and validity bounds hoisted: the r02h source page showed ~120
     // instructions per sub-batch and warp for 24 FMA + 6 stores (cvta sequences, 64-bit store addresses rebuilt from the
@@ -395,7 +374,6 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
     int prev_tile = -1;
     int wv0 = 0, nvalid = 0;
     float T0 = 0.f, T1 = 0.f, T2 = 0.f, sm = 0.f;
-    if(dbg && ew == 0 && lane == 0) dbg[32] = clock64();
     for(int k = 0; k < nit; k++)
     {
       const int item = it0 + k;
@@ -430,24 +408,18 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
       }
       // ---- drain the rest accumulators of this item: 24 frames x (x, y, z), pre-multiplied by scale / sum w ----
       float R[3][FR_WARP];
-      if(!TC3_OFF(512)) TC3_TIMED(w_pfull, ptx::mbar_wait_a(a_pfull, k & 1));
+      ptx::mbar_wait_a(a_pfull, k & 1);
       ptx::tc_fence_after();
 #pragma unroll
       for(int c = 0; c < 3; c++)
       {
-        if(DBG && (p.dbg_mode & 16))
-        {
-#pragma unroll
-          for(int i = 0; i < FR_WARP; i++) R[c][i] = 1.f;
-          continue;
-        }
         ptx::tmem_ld_x16(lane_taddr + c * NF + fp * FR_WARP, R[c]);
         ptx::tmem_ld_x8p(lane_taddr + c * NF + fp * FR_WARP + 16, R[c] + 16);
       }
       ptx::tmem_ld_wait();
       ptx::tc_fence_before();
       __syncwarp();
-      if(lane == 0 && !TC3_OFF(512)) ptx::mbar_arrive_a(a_rest);
+      if(lane == 0) ptx::mbar_arrive_a(a_rest);
       {
         const float s = sp * sm;
 #pragma unroll
@@ -473,25 +445,16 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
           tr[t][1] = __shfl_sync(0xffffffffu, try_, sb * EPI_FR + t);
           tr[t][2] = __shfl_sync(0xffffffffu, trz, sb * EPI_FR + t);
         }
-        if(!TC3_OFF(256)) TC3_TIMED(w_mfull, ptx::mbar_wait_a(a_mfull + 8 * h, (sb >> 1) & 1)); // 6 ring rounds per item: the parity does not depend on the item
+        ptx::mbar_wait_a(a_mfull + 8 * h, (sb >> 1) & 1); // 6 ring rounds per item: the parity does not depend on the item
         ptx::tc_fence_after();
         float M[EPI_FR * kXformFloats];
         const uint32_t mcol = lane_taddr + COL_M + h * SUBN + fp * (EPI_FR * kXformFloats);
-        if(DBG && (p.dbg_mode & 1))
-        {
-#pragma unroll
-          for(int i = 0; i < EPI_FR * kXformFloats; i++) M[i] = 1.f + i;
-        }
-        else
-        {
-          ptx::tmem_ld_x16(mcol, M);
-          ptx::tmem_ld_x8p(mcol + 16, M + 16);
-        }
+        ptx::tmem_ld_x16(mcol, M);
+        ptx::tmem_ld_x8p(mcol + 16, M + 16);
         ptx::tmem_ld_wait();
         ptx::tc_fence_before();
         __syncwarp();
-        if(lane == 0 && !TC3_OFF(256)) ptx::mbar_arrive_a(a_mempty + 8 * h); // the MMA warp may overwrite this matrix buffer
-        if(TC3_OFF(128)) continue;
+        if(lane == 0) ptx::mbar_arrive_a(a_mempty + 8 * h); // the MMA warp may overwrite this matrix buffer
 #pragma unroll
         for(int t = 0; t < EPI_FR; t++)
         {
@@ -500,52 +463,20 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
           const float ox = fmaf(m[0], rx, fmaf(m[1], ry, fmaf(m[2], rz, fmaf(m[3], sm, tr[t][0]))));
           const float oy = fmaf(m[4], rx, fmaf(m[5], ry, fmaf(m[6], rz, fmaf(m[7], sm, tr[t][1]))));
           const float oz = fmaf(m[8], rx, fmaf(m[9], ry, fmaf(m[10], rz, fmaf(m[11], sm, tr[t][2]))));
-          if constexpr(EPI == 0)
+          // no staging: three 4-byte streaming stores per vertex and frame (a warp's 32 vertices are 384 contiguous
+          // bytes; L2 merges the sectors).  Measured +2.4 % against staged float2 stores: the kernel is bound by
+          // shared-memory bandwidth (UMMA operand reads + TMA writes), which the staging round trip competes for.
+          float * o = outl + static_cast<size_t>((sb * SUBF + t) * fstride);
+          if(sb * SUBF + t < nfv)
           {
-            const uint32_t sa = my_stg + (t * 96 + lane * 3) * 4;
-            ptx::sts32(sa, ox);
-            ptx::sts32(sa + 4, oy);
-            ptx::sts32(sa + 8, oz);
-          }
-          else
-          {
-            // no staging: three 4-byte streaming stores per vertex and frame (a warp's 32 vertices are 384 contiguous
-            // bytes; L2 merges the sectors).  Measured +2.4 % against the staged float2 stores: the kernel is bound by
-            // shared-memory bandwidth (UMMA operand reads + TMA writes), which the staging round trip competes for.
-            float * o = outl + static_cast<size_t>((sb * SUBF + t) * fstride);
-            if(sb * SUBF + t < nfv && (!DBG || !(p.dbg_mode & 2) || ox == 1.2345e30f))
-            {
-              __stcs(o, ox);
-              __stcs(o + 1, oy);
-              __stcs(o + 2, oz);
-            }
+            __stcs(o, ox);
+            __stcs(o + 1, oy);
+            __stcs(o + 2, oz);
           }
         }
-        if constexpr(EPI != 0) continue;
-        __syncwarp();
-        // each frame's 32 vertices are 384 contiguous bytes: 8-byte coalesced streaming stores
-#pragma unroll
-        for(int i = 0; i < EPI_FR * 48 / 32; i++)
-        {
-          const int idx = 32 * i + lane; // float2 index over EPI_FR frames x 48
-          const int t = idx / 48;
-          const int w2 = idx - 48 * t;
-          const int f = f0 + sb * SUBF + fp * EPI_FR + t;
-          const float2 val = ptx::lds64(my_stg + idx * 8);
-          if(f < p.B && 2 * w2 < 3 * nvalid)
-            __stcs(reinterpret_cast<float2 *>(outp + (static_cast<size_t>(sb * SUBF + t) * p.V) * 3) + w2, val);
-        }
-        __syncwarp();
       }
     }
-    if(dbg && (ew == 0 || ew == 15) && lane == 0)
-    {
-      if(ew == 0) dbg[33] = clock64();
-      dbg[70 + (ew ? 2 : 0)] = w_pfull, dbg[71 + (ew ? 2 : 0)] = w_mfull;
-    }
   }
-#undef TC3_TIMED
-#undef TC3_OFF
   ptx::tc_fence_before();
   __syncthreads();
   if(warp == 1) ptx::tmem_dealloc<TMEM_COLS>(tmem_base);
@@ -562,25 +493,34 @@ size_t tc3_frame_operand_bytes(int64_t batch)
   return align_up(2 * bpad * tc3::KP * sizeof(__half)) + align_up(2 * bpad * kXformFloats * tc3::KJ * sizeof(__half));
 }
 
-// builds the stage images of the fp16 split basis (scaled like the tc2 copy); called once from smplpp_model_create
-int tc3_prepare_model(ModelDev & d)
+// gate of the tcgen05 kernels (K2''' and lbs_tc_kernel): a CC 10.x device, the driver's tensor-map encoder and an even
+// V >= 128.  Builds the stage images of the fp16 split basis; called once from smplpp_model_create
+int tc3_prepare_model(ModelDev & d, float basis_max_abs)
 {
   d.tc3_ready = false;
-  if(!d.tc2_ready) return SMPLPP_OK;
-  const long long n = static_cast<long long>(d.tc2_tiles) * 3 * tc3::MV * tc3::KP;
+  int dev = 0, major = 0;
+  SB_CUDA(cudaGetDevice(&dev));
+  SB_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
+  SB_CUDA(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, dev));
+  if(major != 10 || !encode_fn() || (d.V & 1) || d.V < tc3::MV || d.sm_count <= 0) return SMPLPP_OK;
+  const int ntiles = (d.V + tc3::MV - 1) / tc3::MV;
+  // largest power of two that keeps |basis| 2^e <= 1024: lo = x - hi stays a normal fp16 for all but tiny entries
+  int e = 0;
+  if(basis_max_abs > 0.f)
+  {
+    while(basis_max_abs * ldexpf(1.f, e + 1) <= 1024.f && e < 24) e++;
+    while(basis_max_abs * ldexpf(1.f, e) > 1024.f && e > -24) e--;
+  }
+  d.tc3_basis_exp = e;
+  const long long n = static_cast<long long>(ntiles) * 3 * tc3::MV * tc3::KP;
   SB_CUDA(cudaMalloc(&d.basis_img16, static_cast<size_t>(2) * n * sizeof(__half)));
-  basis_image_f16_kernel<<<static_cast<unsigned>((n + 255) / 256), 256>>>(d.basis, d.V, d.tc2_tiles, ldexpf(1.f, d.tc2_basis_exp),
+  basis_image_f16_kernel<<<static_cast<unsigned>((n + 255) / 256), 256>>>(d.basis, d.V, ntiles, ldexpf(1.f, e),
                                                                          static_cast<uint8_t *>(d.basis_img16));
   SB_LAUNCHED();
   SB_CUDA(cudaDeviceSynchronize());
-  SB_CUDA(cudaFuncSetAttribute(blend_skin_tc3_kernel<2, 6, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc3::Layout<2, 6, 1>::SMEM_BYTES));
-  SB_CUDA(cudaFuncSetAttribute(blend_skin_tc3_kernel<2, 6, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc3::Layout<2, 6, 1>::SMEM_BYTES));
-  SB_CUDA(cudaFuncSetAttribute(blend_skin_tc3_kernel<3, 3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc3::Layout<3, 3, 1>::SMEM_BYTES));
-  SB_CUDA(cudaFuncSetAttribute(blend_skin_tc3_kernel<2, 6, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc3::Layout<2, 6, 0>::SMEM_BYTES));
-  int dev = 0;
-  SB_CUDA(cudaGetDevice(&dev));
-  SB_CUDA(cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, dev));
-  d.tc3_ready = d.sm_count > 0;
+  SB_CUDA(cudaFuncSetAttribute(blend_skin_tc3_kernel<2, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc3::Layout<2, 6>::SMEM_BYTES));
+  d.tc3_tiles = ntiles;
+  d.tc3_ready = true;
   return SMPLPP_OK;
 }
 
@@ -611,10 +551,10 @@ int launch_blend_skin_tc3(const ModelDev & d, cudaStream_t st, int B, const floa
   p.V = d.V;
   p.B = B;
   p.Bpad = Bpad;
-  p.ntiles = d.tc2_tiles;
+  p.ntiles = d.tc3_tiles;
   p.nfb = Bpad / tc3::NF;
   p.nitems = p.ntiles * p.nfb;
-  p.scale_p = ldexpf(1.f, -(d.tc2_basis_exp + tc3::COEF_EXP));
+  p.scale_p = ldexpf(1.f, -(d.tc3_basis_exp + tc3::COEF_EXP));
   p.scale_m = ldexpf(1.f, -(tc3::W_EXP + tc3::G_EXP));
   p.img_a = static_cast<const uint8_t *>(d.basis_img16);
   p.img_b = img_b;
@@ -624,47 +564,9 @@ int launch_blend_skin_tc3(const ModelDev & d, cudaStream_t st, int B, const floa
   p.wsum = d.lbs_wsum;
   p.theta = theta;
   p.out = out;
-  int grid = p.nitems < d.sm_count ? p.nitems : d.sm_count;
-  static const int grid_env = getenv("SMPLPP_TC3_GRID") ? atoi(getenv("SMPLPP_TC3_GRID")) : 0;
-  static const int ring_env = getenv("SMPLPP_TC3_RING") ? atoi(getenv("SMPLPP_TC3_RING")) : 0;
-  if(grid_env > 0 && grid_env < grid) grid = grid_env;
-  static const bool dbg_on = getenv("SMPLPP_TC3_DBG") != nullptr;
-  p.dbg = nullptr;
-  p.dbg_mode = dbg_on ? atoi(getenv("SMPLPP_TC3_DBG")) >> 1 : 0; // SMPLPP_TC3_DBG = 1 + 2 * mode mask
-  if(dbg_on)
-  {
-    SB_CUDA(cudaMalloc(&p.dbg, static_cast<size_t>(grid) * 256 * sizeof(long long)));
-    SB_CUDA(cudaMemsetAsync(p.dbg, 0, static_cast<size_t>(grid) * 256 * sizeof(long long), st));
-  }
-  if(ring_env == 1) // SMPLPP_TC3_RING: alternatives kept for measurement (3 stages + 3 transform slots; staged stores)
-    blend_skin_tc3_kernel<3, 3, 1><<<grid, tc3::THREADS, tc3::Layout<3, 3, 1>::SMEM_BYTES, st>>>(p);
-  else if(ring_env == 2)
-    blend_skin_tc3_kernel<2, 6, 0><<<grid, tc3::THREADS, tc3::Layout<2, 6, 0>::SMEM_BYTES, st>>>(p);
-  else if(dbg_on)
-    blend_skin_tc3_kernel<2, 6, 1, true><<<grid, tc3::THREADS, tc3::Layout<2, 6, 1>::SMEM_BYTES, st>>>(p);
-  else
-    blend_skin_tc3_kernel<2, 6, 1><<<grid, tc3::THREADS, tc3::Layout<2, 6, 1>::SMEM_BYTES, st>>>(p);
+  const int grid = p.nitems < d.sm_count ? p.nitems : d.sm_count;
+  blend_skin_tc3_kernel<2, 6><<<grid, tc3::THREADS, tc3::Layout<2, 6>::SMEM_BYTES, st>>>(p);
   SB_LAUNCHED();
-  if(dbg_on)
-  {
-    SB_CUDA(cudaStreamSynchronize(st));
-    std::vector<long long> h(static_cast<size_t>(grid) * 256);
-    SB_CUDA(cudaMemcpy(h.data(), p.dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-    cudaFree(p.dbg);
-    for(int cta : {0, grid / 2})
-    {
-      const long long * t = h.data() + static_cast<size_t>(cta) * 256;
-      fprintf(stderr, "[tc3 dbg] cta %d: first GEMM 1 issued +%lld | items", cta, t[1] - t[0]);
-      for(int k = 0; k < 30 && t[2 + k]; k++) fprintf(stderr, " %lld", t[2 + k] - (k ? t[1 + k] : t[1]));
-      fprintf(stderr, " | epilogue %lld .. %lld\n", t[32] - t[0], t[33] - t[0]);
-      fprintf(stderr, "   stage loads issued (K-block 0..13):");
-      for(int i = 0; i < 14; i++) fprintf(stderr, " %lld", t[34 + i] - t[0]);
-      fprintf(stderr, "\n   stage seen full by the MMA thread:  ");
-      for(int i = 0; i < 14; i++) fprintf(stderr, " %lld", t[48 + i] - t[0]);
-      fprintf(stderr, "\n   GEMM 1 issuer: total %lld cycles, blocked on stage %lld, drain %lld | GEMM 2 issuer: total %lld, blocked on transforms %lld, matrix buffer %lld | epilogue warp 0 / 15 blocked on rest accumulators %lld / %lld, on matrices %lld / %lld\n",
-              t[69] - t[0], t[64], t[67], t[68] - t[0], t[65], t[66], t[70], t[72], t[71], t[73]);
-    }
-  }
   return SMPLPP_OK;
 }
 } // namespace sb

@@ -29,17 +29,13 @@ constexpr int EPI_FR = 2;                        // frames of a sub-batch handle
 constexpr int FR_WARP = NSUB * EPI_FR;           // 24 frames of an item per epilogue warp
 constexpr int CTRL_WARPS = 4;                     // one warpgroup: producer, MMA issuer, two idle
 constexpr int THREADS = 32 * (CTRL_WARPS + EPI_WARPS);
-constexpr int STG_FLOATS = EPI_FR * 32 * 3;      // per warp: 2 frames x 32 vertices x 3
-constexpr int STG_BYTES = EPI_WARPS * STG_FLOATS * 4;
-// shared memory: [ST GEMM 1 stages][GS transform sub-batch slots][output staging][barriers]
-template<int ST, int GS, int EPI>
+// shared memory: [ST GEMM 1 stages][GS transform sub-batch slots][barriers]
+template<int ST, int GS>
 struct Layout
 {
   static constexpr int OFF_G = ST * STAGE;
-  static constexpr int OFF_STG = OFF_G + GS * G_STAGE;
-  static constexpr int OFF_BAR = OFF_STG + (EPI == 0 ? STG_BYTES : 0); // only the staged epilogue needs the staging area
+  static constexpr int OFF_BAR = OFF_G + GS * G_STAGE;
   static constexpr int SMEM_BYTES = 1024 + OFF_BAR + 512;
-  static_assert(OFF_STG % 1024 == 0, "swizzle atoms stay aligned");
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
 };
 constexpr int TMEM_COLS = 512;

@@ -35,6 +35,21 @@ def test_struct_layouts_match_header():
     assert C.sizeof(capi.VposerDesc) == 6 * 8
 
 
+def test_set_forward_variant_codes(lib):
+    """smplpp_set_forward_variant accepts exactly the codes include/smplpp_b200.h documents; any other code is
+    refused with the library's error text instead of being mapped to some other implementation."""
+    documented = [0, 1, 3, 6, 200, 201, 202, 300, 301, 400, 401, 402, 410, 411, 420, 421, 422]
+    try:
+        for code in documented:
+            assert lib.smplpp_set_forward_variant(code) == 0, code
+        for code in (2, 4, 5, 7, 100, 101, 203):
+            assert lib.smplpp_set_forward_variant(code) == -1, code
+            assert "unknown forward variant" in lib.smplpp_last_error().decode(), code
+    finally:
+        for code in (0, 202, 300, 400, 410, 420):  # the defaults
+            assert lib.smplpp_set_forward_variant(code) == 0
+
+
 def test_no_cpu_fallback(lib, params):
     import torch
     from smplpp_b200 import api

@@ -71,7 +71,7 @@ def test_kat_linear_blend_skinning(kat):
 
 # ---- full model: golden vectors of the compiled reference ----
 
-@pytest.mark.parametrize("variant", [1, 2, 3, 4, 5, 6])
+@pytest.mark.parametrize("variant", [1, 3, 6])
 def test_forward_vs_reference_golden(smpl_gpu, golden_forward, variant):
     from smplpp_b200 import capi
     g = golden_forward
@@ -86,16 +86,15 @@ def test_forward_vs_reference_golden(smpl_gpu, golden_forward, variant):
     assert np.abs(v - g["vertices"]).max() <= TOL_VERTEX_M
     assert np.abs(j - g["joints"]).max() <= TOL_VERTEX_M
     assert np.abs(rest - g["rest_shape"]).max() <= TOL_VERTEX_M
-    # in practice the fp32 FFMA path and the tcgen05 3xTF32 path sit well below the stated tolerance; 3xBF16 carries
-    # the 2^-17 split residual of both operands (DESIGN.md 4.1)
-    assert np.abs(v - g["vertices"]).max() < (5e-6 if variant == 4 else 2e-6)
+    # in practice the fp32 FFMA path and the tcgen05 fp16 split-precision path sit well below the stated tolerance
+    assert np.abs(v - g["vertices"]).max() < 2e-6
 
 
-@pytest.mark.parametrize("variant", [2, 4, 5, 6])
-@pytest.mark.parametrize("batch", [1, 127, 300])
+@pytest.mark.parametrize("variant", [6])
+@pytest.mark.parametrize("batch", [1, 2, 8, 9, 95, 96, 97, 127, 191, 192, 193, 300])
 def test_forward_tensor_core_variants_match_ffma(smpl_gpu, variant, batch):
-    """Ragged frame counts through the tcgen05 kernel (128-frame tiles, 32-frame transform windows) against the
-    FFMA kernel on the same inputs, every frame and vertex."""
+    """Ragged frame counts through the tcgen05 kernel (96-frame blocks, 8-frame transform sub-batches, frame pairs
+    per epilogue warp) against the FFMA kernel on the same inputs, every frame and vertex."""
     from smplpp_b200 import capi, synth
     beta, theta = synth.make_forward_inputs(batch, 77 + batch)
     out = {}
@@ -107,7 +106,7 @@ def test_forward_tensor_core_variants_match_ffma(smpl_gpu, variant, batch):
         finally:
             capi.check(capi.lib().smplpp_set_forward_variant(0))
     assert np.isfinite(out[variant]).all()
-    assert np.abs(out[variant] - out[1]).max() < (5e-6 if variant == 4 else 1e-6)
+    assert np.abs(out[variant] - out[1]).max() < 1e-6
 
 
 @pytest.mark.parametrize("batch", [2000, 4096 + 37])
