@@ -106,6 +106,11 @@ struct ModelDev
   // tcgen05 blend + skinning (skin_tc3.cu): fp16 hi | lo split basis scaled by 2^tc3_basis_exp.  tc3_ready also
   // gates the tcgen05 standalone skinning kernel (lbs_tc.cu).
   void * basis_img16 = nullptr; // [tile][K-block][hi | lo][plane][128][32 fp16]: SWIZZLE_64B stage images
+  // the two 16-slot joint windows of the skinning product (tc3_layout.cuh): slot s (window s / 16) holds joint
+  // tc3_slot_joint[s] or -1; a joint in both windows has its primary slot (tc3_joint_slot) in window 0
+  int8_t tc3_slot_joint[32] = {};
+  int8_t tc3_joint_slot[kJoints] = {};
+  uint8_t * tc3_tile_mode = nullptr; // (tc3_tiles) per 128-vertex tile: 0 / 1 = its joints fit window 0 / 1, 2 = both
   int tc3_basis_exp = 0;
   int tc3_tiles = 0;
   bool tc3_ready = false;

@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(kChainWarps * 32)
                       const float * __restrict__ joint_shape, int B, const float * __restrict__ beta,
                       long long beta_stride, const float * __restrict__ theta, float * __restrict__ coef,
                       float * __restrict__ xforms, float * __restrict__ joints_out, float * __restrict__ xforms44_out,
-                      uint8_t * __restrict__ img_b, uint8_t * __restrict__ img_g, int Bpad)
+                      uint8_t * __restrict__ img_b, uint8_t * __restrict__ img_g, int Bpad, tc3::WindowMap wmap)
 {
   __shared__ float sG[kChainWarps][kJoints][12];
   __shared__ float sJ[kChainWarps][kJoints][3];
@@ -82,12 +82,11 @@ __global__ void __launch_bounds__(kChainWarps * 32)
         *reinterpret_cast<uint4 *>(blk + tc3::swz64(o)) = z;
         *reinterpret_cast<uint4 *>(blk + tc3::swz64(tc3::B_PART + o)) = z;
       }
-      uint8_t * blk = img_g + (static_cast<size_t>(fb) * tc3::NSUB + nf / tc3::SUBF) * tc3::G_STAGE;
       for(int c = lane; c < kXformFloats * 4; c += 32)
       {
-        const uint32_t o = static_cast<uint32_t>(((nf % tc3::SUBF) * kXformFloats + c / 4) * tc3::ROWB + (c % 4) * 16);
-        *reinterpret_cast<uint4 *>(blk + tc3::swz64(o)) = z;
-        *reinterpret_cast<uint4 *>(blk + tc3::swz64(tc3::G_PART + o)) = z;
+        uint8_t * dst = img_g + tc3::g_chunk_offset(b, c / 4, c % 4);
+        *reinterpret_cast<uint4 *>(dst) = z;
+        *reinterpret_cast<uint4 *>(dst + tc3::G_PART) = z;
       }
     }
     return; // whole warp leaves together; only __syncwarp below
@@ -179,9 +178,9 @@ __global__ void __launch_bounds__(kChainWarps * 32)
   }
   if(img_g)
   {
-    // transform stage image of K2''' (row = frame in its 8-frame sub-batch * 12 + element, column = joint, fp16 hi | lo
-    // x 2^4, SWIZZLE_64B): the relative transforms go back to shared memory and every lane writes 16-byte chunks
-    // (8 joints of one element); this replaces a separate pass over the fp32 transforms
+    // transform stage image of K2''' (tc3::g_chunk_offset: row = frame in its 8-frame sub-batch * 12 + element, two
+    // 16-slot joint windows, fp16 hi | lo x 2^4, SWIZZLE_32B): the relative transforms go back to shared memory and
+    // every lane writes 16-byte chunks (8 slots of one element); this replaces a separate pass over the fp32 transforms
     __syncwarp();
     if(lane < kJoints)
     {
@@ -189,21 +188,17 @@ __global__ void __launch_bounds__(kChainWarps * 32)
       for(int e = 0; e < 12; e++) sG[warp][lane][e] = G[e];
     }
     __syncwarp();
-    const long long fb = b / tc3::NF;
-    const int nf = static_cast<int>(b - fb * tc3::NF);
-    uint8_t * blk = img_g + (static_cast<size_t>(fb) * tc3::NSUB + nf / tc3::SUBF) * tc3::G_STAGE;
     for(int c = lane; c < kXformFloats * 4; c += 32)
     {
       const int e = c / 4, cj = c % 4;
       float x[8];
+      int js[8];
+      tc3::chunk_joints(wmap, cj, js);
 #pragma unroll
       for(int jj = 0; jj < 8; jj++)
-      {
-        const int j = cj * 8 + jj;
-        x[jj] = j < kJoints ? sG[warp][j][e] * static_cast<float>(1 << tc3::G_EXP) : 0.f;
-      }
-      const uint32_t o = static_cast<uint32_t>(((nf % tc3::SUBF) * kXformFloats + e) * tc3::ROWB + cj * 16);
-      tc3::split8_store(x, blk + tc3::swz64(o), blk + tc3::swz64(tc3::G_PART + o));
+        x[jj] = js[jj] >= 0 ? sG[warp][js[jj] < 0 ? 0 : js[jj]][e] * static_cast<float>(1 << tc3::G_EXP) : 0.f;
+      uint8_t * dst = img_g + tc3::g_chunk_offset(b, e, cj);
+      tc3::split8_store(x, dst, dst + tc3::G_PART);
     }
   }
   if(coef)
@@ -868,7 +863,8 @@ int launch_pose_chain(const ModelDev & d, cudaStream_t st, int B, const float * 
   uint8_t * img_g = tc3_scratch ? img_b + tc3::img_g_offset(Bpad) : nullptr;
   int grid = (Bpad + kChainWarps - 1) / kChainWarps;
   pose_chain_kernel<<<grid, kChainWarps * 32, 0, st>>>(make_topo(d), d.joint_template, d.joint_shape, B, beta,
-                                                       beta_stride, theta, coef, xforms, joints, xforms44, img_b, img_g, Bpad);
+                                                       beta_stride, theta, coef, xforms, joints, xforms44, img_b, img_g, Bpad,
+                                                       tc3::window_map(d));
   SB_LAUNCHED();
   return SMPLPP_OK;
 }

@@ -26,7 +26,7 @@ int launch_blend_skin_ffma(const ModelDev & d, cudaStream_t st, int B, const flo
 // K2''' (skin_tc3.cu): fp16 split-precision blend AND skinning matrices on tcgen05 in a persistent CTA per SM; GEMM 1 of
 // item i+1 runs under GEMM 2 + epilogue of item i.  tc3_prepare_model sets d.tc3_ready when the device and the model can
 // run it; basis_max_abs is the largest pose / shape basis entry
-int tc3_prepare_model(ModelDev & d, float basis_max_abs);
+int tc3_prepare_model(ModelDev & d, float basis_max_abs, const float * weights);
 void tc3_release_model(ModelDev & d);
 size_t tc3_frame_operand_bytes(int64_t batch);
 // images_ready: the scratch area already holds the stage images (written by K1); else they are built from coef / xforms

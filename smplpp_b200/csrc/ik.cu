@@ -1854,6 +1854,7 @@ extern "C" int smplpp_tasks_create(const smplpp_model_t * model, int32_t n, cons
   t->sub.basis_img16 = nullptr;
   t->sub.tc3_ready = false;
   t->sub.tc3_tiles = 0;
+  t->sub.tc3_tile_mode = nullptr;
   t->sub.faces = nullptr, t->sub.adj_offset = nullptr, t->sub.adj_faces = nullptr;
   t->sub_corner = t->sub;
   t->sub_corner.V = nCorner;

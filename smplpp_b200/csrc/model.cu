@@ -246,7 +246,7 @@ extern "C" int smplpp_model_create(const smplpp_model_desc * desc, smplpp_model_
     float mx = 0.f; // largest pose / shape basis entry (the template column stays out of the tensor-core product)
     for(size_t r = 0; r < static_cast<size_t>(3) * V; r++)
       for(int k = 0; k < kPoseDim + kShapeDim; k++) mx = std::max(mx, std::fabs(m->h_basis[r * kBlendK + k]));
-    if(tc3_prepare_model(d, mx) != SMPLPP_OK) return SMPLPP_ERR_CUDA;
+    if(tc3_prepare_model(d, mx, m->h_weights.data()) != SMPLPP_OK) return SMPLPP_ERR_CUDA;
   }
   *out = guard.release();
   return SMPLPP_OK;

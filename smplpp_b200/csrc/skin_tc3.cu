@@ -5,7 +5,7 @@
 // T + S + P (src/JointRegression.cpp:551-565) and LinearBlendSkinning::skinning (src/LinearBlendSkinning.cpp:445-553).
 //
 //   rest[v,f]   = T[v] + sum_k basis[v,k] coef[f,k]                 GEMM 1: (128 vertices x 3 planes) x 96 frames, K = 224
-//   M[v,f]      = sum_j W[v,j] G'[f,j]  (3x4 per vertex and frame)  GEMM 2: 128 vertices x (8 frames x 12), K = 24 -> 32
+//   M[v,f]      = sum_j W[v,j] G'[f,j]  (3x4 per vertex and frame)  GEMM 2: 128 vertices x (8 frames x 12), K = 16 or 32
 //   vert[v,f]   = M[v,f] [rest; 1] / sum_j W[v,j] + trans[f]        epilogue: 12 FMA per vertex and frame
 //
 // Work and pipeline (DESIGN.md 4.1 has the measurements):
@@ -13,24 +13,31 @@
 //   * when GEMM 1 of an item completes, the sixteen epilogue warps DRAIN its 288 accumulator columns into registers
 //     (72 per thread, pre-scaled by 1 / sum_j W), which frees the TMEM columns: one thread then issues the 126 MMAs of
 //     the NEXT item's GEMM 1 while another issues the 12 sub-batches of this item's GEMM 2;
-//   * two TMA producer threads, one per ring (2 x 60 KB GEMM 1 stages, 6 x 12 KB transform sub-batches), so neither
+//   * joint windows: the model's 24 joints are covered by two 16-slot windows (chosen from its weights at create time).
+//     A vertex tile whose joints all sit in one window runs GEMM 2 at K = 16 (3 MMAs per sub-batch, 6 KB of transforms);
+//     any other tile runs both windows (6 MMAs, 12 KB), its weights in each joint's primary slot only.  Exact: the
+//     dropped products multiply zero weights;
+//   * two TMA producer threads, one per ring (2 x 60 KB GEMM 1 stages, 6 x 6 KB transform window slots), so neither
 //     ring can starve the other;
 //   * the frames of a 96-frame block are permuted in the fp16 coefficient operand so that the 24 frames an epilogue
 //     warp owns are 24 adjacent accumulator columns (6 tcgen05.ld per drain instead of 36).
 //   * every operand tile is stored in global memory as the exact (SWIZZLE_64B) shared-memory image of its pipeline
 //     stage, so a stage is two contiguous cp.async.bulk copies (48 KB basis + 12 KB coefficients) and a transform
-//     sub-batch is one (12 KB): no tensor maps, a handful of large copies per item.
+//     sub-batch is one (6 or 12 KB, SWIZZLE_32B): no tensor maps, a handful of large copies per item.
 // Precision: both GEMMs are fp32 in the reference.  Every operand is split into fp16 hi + lo (power-of-two pre-scaled
 // so that lo stays a normal fp16) and three products are accumulated in fp32 TMEM, hi.hi + lo.hi + hi.lo (~2^-22
 // relative).  The ~1 m template stays out of GEMM 1 and is added in fp32.
 //
 // TMEM (512 columns): [0,288) rest accumulators (x | y | z planes x 96 frames), [288,480) two 96-column buffers of
-// skinning matrices (8 frames x 12), [480,512) the W tile (A operand of GEMM 2, fp16 hi | lo).
+// skinning matrices (8 frames x 12), [480,512) the W tile (A operand of GEMM 2: window w at 480 + 16 w, fp16 hi | lo).
 // warp 0: TMA producer of the GEMM 1 stages | warp 1: TMEM allocator + issuer of GEMM 2 | warp 2: TMA producer of the transform
 // sub-batches | warp 3: issuer of GEMM 1 (the first warpgroup hands its registers back with setmaxnreg) | warps 4-19: epilogue,
 // 112 registers each (four per TMEM lane quadrant, one per frame pair of an 8-frame sub-batch).
 #include <cuda.h>
 #include <cuda_fp16.h>
+
+#include <algorithm>
+#include <vector>
 
 #include "forward.cuh"
 #include "skin_common.cuh"
@@ -47,13 +54,43 @@ struct Params
   float scale_p, scale_m;       // 2^-(basis_exp + COEF_EXP), 2^-(W_EXP + G_EXP)
   const uint8_t * img_a;        // [tile][K-block][part][plane][128][64 B]   stage image of the fp16 basis
   const uint8_t * img_b;        // [frame block][K-block][part][96][64 B]   stage image of the fp16 coefficients
-  const uint8_t * img_g;        // [frame block][sub-batch][part][96][64 B] stage image of the fp16 transforms
+  const uint8_t * img_g;        // [frame block][sub-batch][window][part][96][32 B] stage image of the fp16 transforms
+  const uint8_t * tile_mode;    // (ntiles) 0 / 1: the tile's joints fit window 0 / 1, 2: both windows
   const float * basis;          // (3 Vpad, 224): column 217 = template
   const float * weights;        // (V, 24) dense
   const float * wsum;           // (Vpad)
   const float * theta;          // (B, 25, 3): row 0 = root translation
   float * out;                  // (B, V, 3)
+  WindowMap wmap;               // transform-image slot -> joint
+  uint32_t primary;             // bit s: slot s is the primary slot of its joint (W tile of a both-window tile)
 };
+
+// One vertex's row of the dense skinning weights -> the W tile (A operand of GEMM 2) in TMEM: lane = vertex, window w
+// at taddr + 16 w (8 hi | 8 lo packed fp16x2 columns).  A window tile (mode 0 / 1) writes its window's joints; a
+// both-window tile (mode 2) puts every joint in its primary slot only, so a joint of both windows counts once.  The
+// caller follows with tmem_st_wait + tcgen05.fence::before_thread_sync before signalling the MMA warp.
+__device__ __forceinline__ void store_w_windows(const float * __restrict__ wrow, uint32_t taddr, const WindowMap wmap,
+                                                uint32_t primary, int mode)
+{
+  uint32_t c[NWIN][KW]; // [window][hi 8 | lo 8]
+#pragma unroll
+  for(int i = 0; i < KJ / 2; i++)
+  {
+    float x[2];
+#pragma unroll
+    for(int h = 0; h < 2; h++)
+    {
+      const int s = 2 * i + h, j = wmap.joint[s];
+      const bool keep = j >= 0 && (mode == 2 ? ((primary >> s) & 1u) != 0 : s / KW == mode);
+      x[h] = keep ? __ldg(wrow + (j < 0 ? 0 : j)) * static_cast<float>(1 << W_EXP) : 0.f;
+    }
+    const float ah = __half2float(__float2half_rn(x[0])), bh = __half2float(__float2half_rn(x[1]));
+    c[i / (KW / 2)][i % (KW / 2)] = skin::pack_half2(ah, bh);
+    c[i / (KW / 2)][KW / 2 + i % (KW / 2)] = skin::pack_half2(x[0] - ah, x[1] - bh);
+  }
+  ptx::tmem_st_x16(taddr, c[0]);
+  ptx::tmem_st_x16(taddr + KW, c[1]);
+}
 
 } // namespace tc3
 
@@ -79,11 +116,11 @@ __global__ void basis_image_f16_kernel(const float * __restrict__ basis, int V, 
 }
 
 // per-call operands: coef (B,224) fp32 -> img_b (rows of every 96-frame block permuted by coef_row, x 2^6);
-// xforms (B,24,12) fp32 -> img_g (row = frame in sub-batch * 12 + element of the 3x4, column = joint, x 2^4).
-// Padding (frames >= B, K >= 217, joints >= 24) is zero-filled.  One thread per 16-byte chunk (8 fp16 of one row:
+// xforms (B,24,12) fp32 -> img_g (row = frame in sub-batch * 12 + element of the 3x4, column = joint slot of the two
+// windows, x 2^4).  Padding (frames >= B, K >= 217, empty slots) is zero-filled.  One thread per 16-byte chunk (8 fp16 of one row:
 // the swizzle moves whole chunks), hi and lo written as one 16-byte store each.
 __global__ void frame_images3_kernel(const float * __restrict__ coef, const float * __restrict__ xforms, int B, int Bpad,
-                                     uint8_t * __restrict__ img_b, uint8_t * __restrict__ img_g)
+                                     uint8_t * __restrict__ img_b, uint8_t * __restrict__ img_g, const tc3::WindowMap wmap)
 {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   constexpr int CK = tc3::KP / 8;   // 28 chunks per coefficient row
@@ -116,17 +153,15 @@ __global__ void frame_images3_kernel(const float * __restrict__ coef, const floa
     const long long row = q / CJ;
     const int e = static_cast<int>(row % kXformFloats);
     const long long f = row / kXformFloats;
+    int js[8];
+    tc3::chunk_joints(wmap, cj, js);
 #pragma unroll
     for(int jj = 0; jj < 8; jj++)
-    {
-      const int j = cj * 8 + jj;
-      x[jj] = (f < B && j < kJoints) ? __ldg(xforms + (f * kJoints + j) * kXformFloats + e) * static_cast<float>(1 << tc3::G_EXP) : 0.f;
-    }
-    const long long fb = f / tc3::NF;
-    const int nf = static_cast<int>(f - fb * tc3::NF);
-    uint8_t * blk = img_g + (static_cast<size_t>(fb) * tc3::NSUB + nf / tc3::SUBF) * tc3::G_STAGE;
-    const uint32_t o = static_cast<uint32_t>(((nf % tc3::SUBF) * kXformFloats + e) * tc3::ROWB + cj * 16);
-    tc3::split8_store(x, blk + tc3::swz64(o), blk + tc3::swz64(tc3::G_PART + o));
+      x[jj] = (f < B && js[jj] >= 0)
+                  ? __ldg(xforms + (f * kJoints + (js[jj] < 0 ? 0 : js[jj])) * kXformFloats + e) * static_cast<float>(1 << tc3::G_EXP)
+                  : 0.f;
+    uint8_t * dst = img_g + tc3::g_chunk_offset(f, e, cj);
+    tc3::split8_store(x, dst, dst + tc3::G_PART);
   }
 }
 
@@ -146,7 +181,7 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
   const uint32_t bar32 = smem32 + OFF_BAR;
   uint64_t * full = bars;                // [STAGES]  TMA -> MMA (GEMM 1 stages)
   uint64_t * empty = full + STAGES;      // [STAGES]  MMA -> TMA
-  uint64_t * g_full = empty + STAGES;    // [GSLOTS]  TMA -> MMA (transform sub-batches)
+  uint64_t * g_full = empty + STAGES;    // [GSLOTS]  TMA -> MMA (transform windows of a sub-batch)
   uint64_t * g_empty = g_full + GSLOTS;  // [GSLOTS]  MMA -> TMA
   uint64_t * m_full = g_empty + GSLOTS;  // [2]       MMA -> epilogue (skinning matrices of a sub-batch)
   uint64_t * m_empty = m_full + 2;       // [2]       epilogue -> MMA
@@ -226,24 +261,27 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
   }
   else if(warp == 2)
   {
-    // ---- producer of the transform sub-batch ring ----
+    // ---- producer of the transform ring: per sub-batch one 6 KB entry (the tile's window) or, for a both-window
+    //      tile, two consecutive entries filled by ONE 12 KB copy signalled on the first (the second barrier gets a
+    //      plain arrival so that every entry completes one phase) ----
     if(ptx::elect_one())
     {
-      const int total_g = nit * NSUB;
-      int sb = 0, fb = it0 % p.nfb;
-      for(int gn = 0; gn < total_g; gn++)
+      int gn = 0, fb = it0 % p.nfb, tile = it0 / p.nfb;
+      for(int k = 0; k < nit; k++)
       {
-        const uint32_t s = static_cast<uint32_t>(gn % GSLOTS);
-        const uint8_t * src = p.img_g + (static_cast<size_t>(fb) * NSUB + sb) * G_STAGE;
-        const uint32_t fbar = bar32 + 8 * (2 * STAGES + s);
-        ptx::mbar_wait_a(bar32 + 8 * (2 * STAGES + GSLOTS + s), ((gn / GSLOTS) & 1) ^ 1);
-        ptx::mbar_expect_tx_a(fbar, G_STAGE);
-        ptx::bulk_load_1d_a(smem32 + OFF_G + s * G_STAGE, src, G_STAGE, fbar);
-        if(++sb == NSUB)
+        const int mode = p.tile_mode[tile], nw = mode == 2 ? 2 : 1;
+        const uint8_t * src = p.img_g + static_cast<size_t>(fb) * NSUB * G_SUB + (mode == 1 ? G_WIN : 0);
+        for(int sb = 0; sb < NSUB; sb++, gn += nw)
         {
-          sb = 0;
-          if(++fb == p.nfb) fb = 0;
+          const uint32_t s = static_cast<uint32_t>(gn % GSLOTS), par = ((gn / GSLOTS) & 1) ^ 1;
+          const uint32_t fbar = bar32 + 8 * (2 * STAGES + s), ebar = bar32 + 8 * (2 * STAGES + GSLOTS + s);
+          ptx::mbar_wait_a(ebar, par);
+          if(nw == 2) ptx::mbar_wait_a(ebar + 8, par);
+          ptx::mbar_expect_tx_a(fbar, nw * G_WIN);
+          ptx::bulk_load_1d_a(smem32 + OFF_G + s * G_WIN, src + static_cast<size_t>(sb) * G_SUB, nw * G_WIN, fbar);
+          if(nw == 2) ptx::mbar_arrive_a(fbar + 8);
         }
+        if(++fb == p.nfb) fb = 0, tile++;
       }
     }
   }
@@ -256,14 +294,17 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
       // Every instruction between two tcgen05.mma is on the critical path of its issuing thread.  ncu's source page of the
       // single-issuer version (r02h) had that thread at 1800 instructions per item for 198 MMAs and blocked on a full
       // tensor queue in only a quarter of its samples: the tensor pipe starved behind the issue loop.  Hence (a) TWO
-      // issuing threads - warp 3 the 126 GEMM 1 MMAs of the next item, warp 1 the 72 GEMM 2 MMAs of this one; the tensor
+      // issuing threads - warp 3 the 126 GEMM 1 MMAs of the next item, warp 1 the 36 (window tile) or 72 (both-window
+      // tile) GEMM 2 MMAs of this one; the tensor
       // queue interleaves them (0.1725 -> 0.1607 ms per launch) - and (b) lean streams: the sub-batches and half K-blocks
       // are unrolled, so that ring slots, parities and operand offsets are compile-time constants; only the stage of a
       // K-block (ring position over all items) and the item parity are run-time values, and barriers are 32-bit shared
       // addresses.  Descriptor = constant high word | (shared address >> 4).
-      static_assert(NSUB % GSLOTS == 0 && ((NSUB / GSLOTS) & 1) == 0, "transform ring: slot and parity of a sub-batch do not depend on the item");
+      static_assert(NSUB % GSLOTS == 0 && ((NSUB / GSLOTS) & 1) == 0 && GSLOTS % 2 == 0,
+                    "transform ring (12 or 24 entries per item): slot and parity of an entry do not depend on the item, "
+                    "and the two entries of a both-window sub-batch are adjacent slots");
       static_assert((NSUB & 3) == 0, "matrix buffers: parity of a sub-batch does not depend on the item");
-      constexpr uint32_t DHI = ptx::smem_desc_hi<ROWB>();
+      constexpr uint32_t DHI = ptx::smem_desc_hi<ROWB>(), DHI_G = ptx::smem_desc_hi<ROWG>();
       const uint32_t smem16 = smem32 >> 4;
       const uint32_t a_full = bar32; // one base register, every other barrier at a compile-time offset
       const uint32_t a_empty = a_full + 8 * STAGES, a_gfull = a_empty + 8 * STAGES, a_gempty = a_gfull + 8 * GSLOTS,
@@ -279,11 +320,30 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
         ptx::umma_f16_ss_lo(tmem_base + c * NF, st16 + ((a_part * A_PART + c * MV * ROWB + ks * 32) >> 4),
                             st16 + ((2 * A_PART + b_part * B_PART + ks * 32) >> 4), DHI, idesc1, acc);
       };
-      // GEMM 2 MMA j (0..5) of a sub-batch: hi.hi, lo.hi, hi.lo with two K = 16 steps each
-      auto g2_mma = [&](uint32_t dm, uint32_t aw, uint32_t sg16, int j) {
-        const int prod = j >> 1, ks = j & 1;
-        const int pa = prod == 1 ? 1 : 0, pb = prod == 2 ? 1 : 0;
-        ptx::umma_f16_ts_lo(dm, aw + pa * (KJ / 2) + ks * 8, sg16 + ((pb * G_PART + ks * 32) >> 4), DHI, idesc2, j != 0 ? 1u : 0u);
+      // GEMM 2 of sub-batch sb (compile-time after unrolling) over nw windows: hi.hi, lo.hi, hi.lo at K = 16 per window.
+      // nw = 1: ring entry sb, aw = the tile's window of the W tile; nw = 2 (both-window tile): entries 2 sb, 2 sb + 1,
+      // whose data the first barrier covers, aw = window 0
+      auto g2_sub = [&](int sb, int nw, uint32_t aw) {
+        const int b = sb & 1, e0 = sb * nw, gs0 = e0 % GSLOTS;
+        ptx::mbar_wait_a(a_gfull + 8 * gs0, (e0 / GSLOTS) & 1);
+        ptx::mbar_wait_a(a_mempty + 8 * b, ((sb >> 1) & 1) ^ 1);
+        ptx::tc_fence_after();
+        const uint32_t dm = tmem_base + COL_M + b * SUBN;
+#pragma unroll
+        for(int w = 0; w < nw; w++)
+        {
+          const uint32_t sg16 = smem16 + ((OFF_G + (gs0 + w) * G_WIN) >> 4);
+#pragma unroll
+          for(int prod = 0; prod < 3; prod++)
+          {
+            const int pa = prod == 1 ? 1 : 0, pb = prod == 2 ? 1 : 0;
+            ptx::umma_f16_ts_lo(dm, aw + w * KW + pa * (KW / 2), sg16 + ((pb * G_PART) >> 4), DHI_G, idesc2,
+                                (w | prod) != 0 ? 1u : 0u);
+          }
+        }
+        ptx::tc_commit_a(a_mfull + 8 * b);
+#pragma unroll
+        for(int w = 0; w < nw; w++) ptx::tc_commit_a(a_gempty + 8 * (gs0 + w));
       };
       // half K-block h (compile-time after unrolling: K-block h / 2, operand half h % 2) of the GEMM 1 whose first K-block
       // has ring position kbn0 (run-time).  The even half waits for the TMA data, the odd half hands the stage back.
@@ -324,32 +384,30 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
           ptx::tc_commit_a(a_pfull);
         }
       }
-      // ---- GEMM 2 issuer (warp 1): the twelve sub-batches of every item, two matrix buffers ----
-      int wcount = 0, prev_tile = -1;
+      // ---- GEMM 2 issuer (warp 1): the twelve sub-batches of every item, two matrix buffers; the tile mode selects
+      //      one of two unrolled streams once per item ----
+      int wcount = 0, prev_tile = -1, mode = 0;
       for(int k = 0; k < (warp == 3 ? 0 : nit); k++)
       {
         const int tile = (it0 + k) / p.nfb;
         if(tile != prev_tile)
         {
+          mode = p.tile_mode[tile];
           ptx::mbar_wait_a(a_wready, wcount & 1);
           ptx::tc_fence_after();
           wcount++;
           prev_tile = tile;
         }
-        const uint32_t aw = tmem_base + COL_W;
-#pragma unroll
-        for(int sb = 0; sb < NSUB; sb++)
+        if(mode == 2)
         {
-          const int b = sb & 1, gs = sb % GSLOTS;
-          ptx::mbar_wait_a(a_gfull + 8 * gs, (sb / GSLOTS) & 1);
-          ptx::mbar_wait_a(a_mempty + 8 * b, ((sb >> 1) & 1) ^ 1);
-          ptx::tc_fence_after();
-          const uint32_t sg16 = smem16 + ((OFF_G + gs * G_STAGE) >> 4);
-          const uint32_t dm = tmem_base + COL_M + b * SUBN;
 #pragma unroll
-          for(int j = 0; j < 6; j++) g2_mma(dm, aw, sg16, j);
-          ptx::tc_commit_a(a_mfull + 8 * b);
-          ptx::tc_commit_a(a_gempty + 8 * gs);
+          for(int sb = 0; sb < NSUB; sb++) g2_sub(sb, 2, tmem_base + COL_W);
+        }
+        else
+        {
+          const uint32_t aw = tmem_base + COL_W + KW * mode;
+#pragma unroll
+          for(int sb = 0; sb < NSUB; sb++) g2_sub(sb, 1, aw);
         }
       }
     }
@@ -387,7 +445,8 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
         if(ew < 4)
         {
           // every MMA that read the previous W tile has completed: this warp has seen m_full of the item's last sub-batch
-          skin::store_w_row_tmem(p.weights + static_cast<size_t>(vc) * kJoints, lane_taddr + COL_W);
+          store_w_windows(p.weights + static_cast<size_t>(vc) * kJoints, lane_taddr + COL_W, p.wmap, p.primary,
+                          p.tile_mode[tile]);
           ptx::tmem_st_wait();
           ptx::tc_fence_before();
           __syncwarp();
@@ -485,6 +544,74 @@ __global__ void __launch_bounds__(tc3::THREADS, 1)
 // ------------------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------------------
+namespace
+{
+// GEMM 1 stages of 60 KB.  Three fit next to the six 6 KB transform slots (222 720 B), but measured slower than two
+// (DESIGN.md 4.1)
+constexpr int kStages = 2;
+
+// The two joint windows of GEMM 2 (K = 16 each) for the skinning weights w (V, 24).  A vertex has at most a few
+// non-zero weights and models number their vertices region by region, so most 128-vertex tiles touch a handful of
+// joints; a tile whose joints all sit in one window needs one K step instead of two.  W0 holds 16 joints, W1 the 8
+// others plus up to 8 joints of W0.  Every W0 is tried (C(24,16) = 735471, in increasing bit order); given W0, W1 takes
+// the joints of the tiles that do not fit W0, largest tile first, while it stays within 16 joints.  The first W0 with
+// the fewest vertices in tiles that fit neither window wins.  Only vertices < V count.
+void choose_windows(const float * w, int V, int8_t (&slot_joint)[tc3::KJ], int8_t (&joint_slot)[kJoints],
+                    std::vector<uint8_t> & mode)
+{
+  const int ntiles = (V + tc3::MV - 1) / tc3::MV;
+  std::vector<uint32_t> tmask(ntiles, 0u);
+  for(int v = 0; v < V; v++)
+    for(int j = 0; j < kJoints; j++)
+      if(w[static_cast<size_t>(v) * kJoints + j] != 0.f) tmask[v / tc3::MV] |= 1u << j;
+  // distinct joint sets with their vertex counts, largest first (ties: first tile first)
+  std::vector<std::pair<uint32_t, int>> sets;
+  for(int t = 0; t < ntiles; t++)
+  {
+    const int nv = std::min(V, (t + 1) * tc3::MV) - t * tc3::MV;
+    auto it = std::find_if(sets.begin(), sets.end(), [&](const std::pair<uint32_t, int> & q) { return q.first == tmask[t]; });
+    if(it == sets.end())
+      sets.emplace_back(tmask[t], nv);
+    else
+      it->second += nv;
+  }
+  std::stable_sort(sets.begin(), sets.end(), [](const std::pair<uint32_t, int> & a, const std::pair<uint32_t, int> & b) {
+    return a.second > b.second;
+  });
+  const uint32_t all = (1u << kJoints) - 1;
+  uint32_t best0 = 0, best1 = 0;
+  long long best_cost = -1;
+  for(uint32_t m0 = (1u << tc3::KW) - 1; m0 <= all;)
+  {
+    uint32_t m1 = all & ~m0;
+    long long cost = 0;
+    for(const auto & q : sets)
+    {
+      if((q.first & ~m0) == 0) continue;
+      const uint32_t u = m1 | q.first;
+      if(__builtin_popcount(u) <= tc3::KW)
+        m1 = u;
+      else
+        cost += q.second;
+    }
+    if(best_cost < 0 || cost < best_cost) best_cost = cost, best0 = m0, best1 = m1;
+    if(cost == 0) break;
+    const uint32_t c = m0 & (~m0 + 1u), r = m0 + c; // next set of 16 bits (Gosper)
+    m0 = (((r ^ m0) >> 2) / c) | r;
+  }
+  int n0 = 0, n1 = tc3::KW;
+  for(int s = 0; s < tc3::KJ; s++) slot_joint[s] = -1;
+  for(int j = 0; j < kJoints; j++)
+  {
+    if(best1 >> j & 1u) slot_joint[n1++] = static_cast<int8_t>(j);
+    if(best0 >> j & 1u) slot_joint[n0++] = static_cast<int8_t>(j);
+    joint_slot[j] = static_cast<int8_t>((best0 >> j & 1u) ? n0 - 1 : n1 - 1);
+  }
+  mode.resize(ntiles);
+  for(int t = 0; t < ntiles; t++) mode[t] = (tmask[t] & ~best0) == 0 ? 0 : (tmask[t] & ~best1) == 0 ? 1 : 2;
+}
+} // namespace
+
 namespace sb
 {
 size_t tc3_frame_operand_bytes(int64_t batch)
@@ -494,8 +621,9 @@ size_t tc3_frame_operand_bytes(int64_t batch)
 }
 
 // gate of the tcgen05 kernels (K2''' and lbs_tc_kernel): a CC 10.x device, the driver's tensor-map encoder and an even
-// V >= 128.  Builds the stage images of the fp16 split basis; called once from smplpp_model_create
-int tc3_prepare_model(ModelDev & d, float basis_max_abs)
+// V >= 128.  Builds the stage images of the fp16 split basis and chooses the joint windows from the host weights
+// (V, 24); called once from smplpp_model_create
+int tc3_prepare_model(ModelDev & d, float basis_max_abs, const float * weights)
 {
   d.tc3_ready = false;
   int dev = 0, major = 0;
@@ -517,8 +645,13 @@ int tc3_prepare_model(ModelDev & d, float basis_max_abs)
   basis_image_f16_kernel<<<static_cast<unsigned>((n + 255) / 256), 256>>>(d.basis, d.V, ntiles, ldexpf(1.f, e),
                                                                          static_cast<uint8_t *>(d.basis_img16));
   SB_LAUNCHED();
+  std::vector<uint8_t> mode;
+  choose_windows(weights, d.V, d.tc3_slot_joint, d.tc3_joint_slot, mode);
+  SB_CUDA(cudaMalloc(&d.tc3_tile_mode, mode.size()));
+  SB_CUDA(cudaMemcpy(d.tc3_tile_mode, mode.data(), mode.size(), cudaMemcpyHostToDevice));
   SB_CUDA(cudaDeviceSynchronize());
-  SB_CUDA(cudaFuncSetAttribute(blend_skin_tc3_kernel<2, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc3::Layout<2, 6>::SMEM_BYTES));
+  SB_CUDA(cudaFuncSetAttribute(blend_skin_tc3_kernel<kStages, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               tc3::Layout<kStages, 6>::SMEM_BYTES));
   d.tc3_tiles = ntiles;
   d.tc3_ready = true;
   return SMPLPP_OK;
@@ -527,7 +660,9 @@ int tc3_prepare_model(ModelDev & d, float basis_max_abs)
 void tc3_release_model(ModelDev & d)
 {
   if(d.basis_img16) cudaFree(d.basis_img16);
+  if(d.tc3_tile_mode) cudaFree(d.tc3_tile_mode);
   d.basis_img16 = nullptr;
+  d.tc3_tile_mode = nullptr;
   d.tc3_ready = false;
 }
 
@@ -544,7 +679,8 @@ int launch_blend_skin_tc3(const ModelDev & d, cudaStream_t st, int B, const floa
   if(!images_ready)
   {
     const long long n = static_cast<long long>(Bpad) * (tc3::KP + kXformFloats * tc3::KJ) / 8; // 16-byte chunks
-    frame_images3_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(coef, xforms, B, Bpad, img_b, img_g);
+    frame_images3_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(coef, xforms, B, Bpad, img_b, img_g,
+                                                                                  tc3::window_map(d));
     SB_LAUNCHED();
   }
   tc3::Params p;
@@ -559,13 +695,17 @@ int launch_blend_skin_tc3(const ModelDev & d, cudaStream_t st, int B, const floa
   p.img_a = static_cast<const uint8_t *>(d.basis_img16);
   p.img_b = img_b;
   p.img_g = img_g;
+  p.tile_mode = d.tc3_tile_mode;
+  p.wmap = tc3::window_map(d);
+  p.primary = 0;
+  for(int j = 0; j < kJoints; j++) p.primary |= 1u << d.tc3_joint_slot[j];
   p.basis = d.basis;
   p.weights = d.weights_dense;
   p.wsum = d.lbs_wsum;
   p.theta = theta;
   p.out = out;
   const int grid = p.nitems < d.sm_count ? p.nitems : d.sm_count;
-  blend_skin_tc3_kernel<2, 6><<<grid, tc3::THREADS, tc3::Layout<2, 6>::SMEM_BYTES, st>>>(p);
+  blend_skin_tc3_kernel<kStages, 6><<<grid, tc3::THREADS, tc3::Layout<kStages, 6>::SMEM_BYTES, st>>>(p);
   SB_LAUNCHED();
   return SMPLPP_OK;
 }

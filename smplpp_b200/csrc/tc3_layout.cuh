@@ -20,21 +20,25 @@ constexpr int B_PART = NF * ROWB;                // 6144
 constexpr int STAGE = 2 * A_PART + 2 * B_PART;   // 61440
 constexpr int SUBF = 8;                          // frames per skinning sub-batch
 constexpr int SUBN = SUBF * kXformFloats;        // 96 = UMMA N of GEMM 2
-constexpr int KJ = skin::KJ;                     // joints padded to two K = 16 steps
-constexpr int G_PART = SUBN * ROWB;              // 6144
-constexpr int G_STAGE = 2 * G_PART;              // 12288
+constexpr int KW = 16;                           // joint slots per window (one K = 16 step of GEMM 2)
+constexpr int NWIN = 2;                          // joint windows per model
+constexpr int KJ = NWIN * KW;                    // 32 slots per transform row
+constexpr int ROWG = KW * 2;                     // bytes of one window's row (one SWIZZLE_32B span = 16 fp16)
+constexpr int G_PART = SUBN * ROWG;              // 3072: one part (hi or lo) of one window of a sub-batch
+constexpr int G_WIN = 2 * G_PART;                // 6144: one window of a sub-batch = one transform ring slot
+constexpr int G_SUB = NWIN * G_WIN;              // 12288: one sub-batch of the transform image
 constexpr int NSUB = NF / SUBF;                  // 12 sub-batches per item
 constexpr int EPI_WARPS = 16;
 constexpr int EPI_FR = 2;                        // frames of a sub-batch handled by one epilogue warp
 constexpr int FR_WARP = NSUB * EPI_FR;           // 24 frames of an item per epilogue warp
 constexpr int CTRL_WARPS = 4;                     // one warpgroup: producer, MMA issuer, two idle
 constexpr int THREADS = 32 * (CTRL_WARPS + EPI_WARPS);
-// shared memory: [ST GEMM 1 stages][GS transform sub-batch slots][barriers]
+// shared memory: [ST GEMM 1 stages][GS transform window slots][barriers]
 template<int ST, int GS>
 struct Layout
 {
   static constexpr int OFF_G = ST * STAGE;
-  static constexpr int OFF_BAR = OFF_G + GS * G_STAGE;
+  static constexpr int OFF_BAR = OFF_G + GS * G_WIN;
   static constexpr int SMEM_BYTES = 1024 + OFF_BAR + 512;
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
 };
@@ -43,8 +47,34 @@ constexpr int COL_M = 3 * NF;                    // 288
 constexpr int COL_W = COL_M + 2 * SUBN;          // 480
 constexpr int TRIPLES = NKB * 6;                 // GEMM 1 = 42 (K-block, product, K-step) triples of 3 MMAs (planes)
 constexpr int COEF_EXP = 6, W_EXP = skin::W_EXP, G_EXP = skin::G_EXP;
-static_assert(COL_W + 2 * (KJ / 2) == TMEM_COLS, "TMEM column map");
-static_assert(STAGE % 1024 == 0 && G_STAGE % 1024 == 0, "swizzle atoms stay aligned");
+static_assert(COL_W + NWIN * KW == TMEM_COLS, "TMEM column map: window w at COL_W + 16 w (8 hi | 8 lo columns)");
+static_assert(STAGE % 1024 == 0 && G_WIN % 1024 == 0 && G_PART % 256 == 0, "swizzle atoms stay aligned");
+
+// The two joint windows of a model (chosen by tc3_prepare_model from its skinning weights): slot s of the transform
+// image belongs to window s / KW and holds joint[s], or zeros for -1.  A joint may sit in both windows.
+struct WindowMap
+{
+  int8_t joint[KJ];
+};
+// joints of slots 8 c .. 8 c + 7 for a run-time c (0..3): selects between constant indices, so that the map (a kernel
+// parameter) is not copied to local memory
+__device__ __forceinline__ void chunk_joints(const WindowMap & m, int c, int (&j)[8])
+{
+#pragma unroll
+  for(int jj = 0; jj < 8; jj++)
+  {
+    j[jj] = m.joint[jj];
+#pragma unroll
+    for(int q = 1; q < KJ / 8; q++) j[jj] = c == q ? m.joint[8 * q + jj] : j[jj];
+  }
+}
+static_assert(sizeof(ModelDev::tc3_slot_joint) == KJ, "slot map of the model");
+inline WindowMap window_map(const ModelDev & d)
+{
+  WindowMap m;
+  for(int s = 0; s < KJ; s++) m.joint[s] = d.tc3_slot_joint[s];
+  return m;
+}
 
 // frame n of a 96-frame block -> row of the block in the fp16 coefficient operand (= accumulator column of GEMM 1):
 // the 24 frames epilogue warp group fp owns (frame pair fp of every 8-frame sub-batch) become adjacent columns
@@ -59,6 +89,21 @@ __host__ __device__ constexpr int coef_row(int n)
 __host__ __device__ constexpr uint32_t swz64(uint32_t o)
 {
   return o ^ (((o >> 7) & 3u) << 4);
+}
+// the same for SWIZZLE_32B (16-byte chunk index XOR bit 7 of the offset), inside a 256-byte aligned region
+__host__ __device__ constexpr uint32_t swz32(uint32_t o)
+{
+  return o ^ (((o >> 7) & 1u) << 4);
+}
+
+// transform image [frame block][sub-batch][window][hi | lo][96 rows][16 slots], SWIZZLE_32B: byte offset of the hi
+// 16-byte chunk with slots 8 c .. 8 c + 7 (c = 0..3, window c / 2) of element e (0..11) of frame f; lo is G_PART further
+__host__ __device__ inline size_t g_chunk_offset(long long f, int e, int c)
+{
+  const long long fb = f / NF;
+  const int nf = static_cast<int>(f - fb * NF);
+  const size_t blk = ((static_cast<size_t>(fb) * NSUB + nf / SUBF) * NWIN + c / 2) * G_WIN;
+  return blk + swz32(static_cast<uint32_t>(((nf % SUBF) * kXformFloats + e) * ROWG + (c % 2) * 16));
 }
 
 // eight consecutive K values of one operand row -> fp16 hi | lo 16-byte chunks at their (swizzled) places

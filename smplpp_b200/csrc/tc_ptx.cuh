@@ -346,8 +346,8 @@ __device__ __forceinline__ void umma_f16_ss(uint32_t d_tmem, uint64_t a_desc, ui
 template<int kRowBytes>
 __host__ __device__ constexpr uint32_t smem_desc_hi()
 {
-  static_assert(kRowBytes == 64 || kRowBytes == 128, "row = one swizzle span");
-  return static_cast<uint32_t>((8 * kRowBytes) >> 4) | (1u << 14) | ((kRowBytes == 128 ? 2u : 4u) << 29);
+  static_assert(kRowBytes == 32 || kRowBytes == 64 || kRowBytes == 128, "row = one swizzle span");
+  return static_cast<uint32_t>((8 * kRowBytes) >> 4) | (1u << 14) | ((kRowBytes == 128 ? 2u : kRowBytes == 64 ? 4u : 6u) << 29);
 }
 __device__ __forceinline__ void umma_f16_ss_lo(uint32_t d_tmem, uint32_t a_lo, uint32_t b_lo, uint32_t desc_hi, uint32_t idesc,
                                                uint32_t accumulate)
@@ -398,13 +398,14 @@ __host__ __device__ constexpr uint32_t make_idesc(bool tf32, int m, int n)
 }
 
 // UMMA shared-memory matrix descriptor for a K-major tile whose rows are exactly one swizzle span wide
-// (64 B -> SWIZZLE_64B, 128 B -> SWIZZLE_128B): 8-row atoms are contiguous, SBO = 8 * row bytes, LBO unused.
+// (32 B -> SWIZZLE_32B, 64 B -> SWIZZLE_64B, 128 B -> SWIZZLE_128B): 8-row atoms are contiguous, SBO = 8 * row bytes,
+// LBO unused.
 //   bits [0,14) address >> 4 | [16,30) LBO >> 4 | [32,46) SBO >> 4 | [46,48) version = 1 | [61,64) layout type
 template<int kRowBytes>
 __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr)
 {
-  static_assert(kRowBytes == 64 || kRowBytes == 128, "row = one swizzle span");
-  constexpr uint64_t layout = kRowBytes == 128 ? 2 : 4;
+  static_assert(kRowBytes == 32 || kRowBytes == 64 || kRowBytes == 128, "row = one swizzle span");
+  constexpr uint64_t layout = kRowBytes == 128 ? 2 : kRowBytes == 64 ? 4 : 6;
   constexpr uint64_t sbo = (8 * kRowBytes) >> 4;
   return static_cast<uint64_t>((smem_addr & 0x3FFFF) >> 4) | (sbo << 32) | (1ull << 46) | (layout << 61);
 }
