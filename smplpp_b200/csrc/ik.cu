@@ -52,6 +52,9 @@ __global__ void task_positions_kernel(const int32_t * __restrict__ faces, const 
   const float * vb = verts + static_cast<size_t>(b) * V * 3;
   const int f = face_idx32 ? face_idx32[i] : static_cast<int>(face_idx[m]);
   const float * w = weights + i * 3;
+  // normals and tangents written out, not through face_normal / corner_normal / tangent_frame (ik_math.cuh): with either
+  // the normal helpers alone or tangent_frame alone in the dphi branch, the normals returned by smplpp_task_positions
+  // changed in the last bits (same instruction mix, other scheduling)
   f3 p = mk3(0.f, 0.f, 0.f), s = mk3(0.f, 0.f, 0.f);
   const bool need_n = offset > 0.f || nrm_out != nullptr;
   for(int c = 0; c < 3; c++)
@@ -92,8 +95,7 @@ __global__ void task_positions_kernel(const int32_t * __restrict__ faces, const 
   pos_out[3 * i] = p.x, pos_out[3 * i + 1] = p.y, pos_out[3 * i + 2] = p.z;
 }
 
-// IkTask::calcTangents (src/IkTask.cpp:33-47): t1 = normalize(v1 - v0), t2 = normalize(((v1 - v0) x (v2 - v0)) x (v1 - v0));
-// out (B, n, 3, 2) like IkTask::tangents_ (columns are the two tangents)
+// IkTask::calcTangents (src/IkTask.cpp:33-47); out (B, n, 3, 2) like IkTask::tangents_ (columns are the two tangents)
 __global__ void task_tangents_kernel(const int32_t * __restrict__ faces, int V, int B, int n,
                                      const long long * __restrict__ face_idx, const int32_t * __restrict__ face_idx32,
                                      const float * __restrict__ verts, float * __restrict__ out)
@@ -103,13 +105,10 @@ __global__ void task_tangents_kernel(const int32_t * __restrict__ faces, int V, 
   const int b = static_cast<int>(i / n), m = static_cast<int>(i % n);
   const float * vb = verts + static_cast<size_t>(b) * V * 3;
   const int f = face_idx32 ? face_idx32[i] : static_cast<int>(face_idx[m]);
-  const f3 v0 = ld3(vb + 3 * faces[3 * f]), v1 = ld3(vb + 3 * faces[3 * f + 1]), v2 = ld3(vb + 3 * faces[3 * f + 2]);
-  const f3 t1r = v1 - v0;
-  const f3 t2r = cross3(cross3(t1r, v2 - v0), t1r);
-  float inv;
-  const f3 t1 = normalize_inv(t1r, inv), t2 = normalize_inv(t2r, inv);
+  f3 t[2];
+  tangent_frame(ld3(vb + 3 * faces[3 * f]), ld3(vb + 3 * faces[3 * f + 1]), ld3(vb + 3 * faces[3 * f + 2]), t);
   float * o = out + 6 * i;
-  o[0] = t1.x, o[1] = t2.x, o[2] = t1.y, o[3] = t2.y, o[4] = t1.z, o[5] = t2.z;
+  o[0] = t[0].x, o[1] = t[1].x, o[2] = t[0].y, o[3] = t[1].y, o[4] = t[0].z, o[5] = t[1].z;
 }
 
 // VPoser state (B,44) -> theta rows 0,1 and 23,24 (node.cpp:761-772); rows 2..22 are written by the decoder
@@ -222,66 +221,10 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
 
   // ---- P1: rotations, their derivatives, joints ----
   if(tid < kJoints)
-  {
-    const int j = tid;
-    rodrigues_grad(s_theta[3 + 3 * j], s_theta[4 + 3 * j], s_theta[5 + 3 * j], s_R + 9 * j, s_dR + 27 * j);
-#pragma unroll
-    for(int k = 0; k < 3; k++)
-    {
-      float acc = p.joint_template[3 * j + k];
-#pragma unroll
-      for(int i = 0; i < kShapeDim; i++)
-      {
-        float js = p.joint_shape[(3 * j + k) * kShapeDim + i];
-        acc = fmaf(js, s_beta[i], acc);
-        if(p.beta_cols) s_JS[(3 * j + k) * kShapeDim + i] = js;
-      }
-      s_Jt[3 * j + k] = acc;
-    }
-  }
+    chain_joint(tid, s_theta, s_beta, p.joint_template, p.joint_shape, p.beta_cols, s_R, s_dR, s_Jt, s_JS);
   __syncthreads();
   // ---- P2a: global transforms level by level (warp 0) ----
-  if(tid < 32)
-  {
-    const int j = tid;
-    const int parent = j < kJoints ? p.topo.parent[j] : -1;
-    const int depth = j < kJoints ? p.topo.depth[j] : -1;
-    for(int d = 0; d <= p.topo.max_depth; d++)
-    {
-      if(depth == d)
-      {
-        const float * R = s_R + 9 * j;
-        float * G = s_G + 12 * j;
-        if(parent < 0)
-        {
-          for(int r = 0; r < 3; r++)
-          {
-            G[4 * r] = R[3 * r], G[4 * r + 1] = R[3 * r + 1], G[4 * r + 2] = R[3 * r + 2];
-            G[4 * r + 3] = s_Jt[3 * j + r];
-          }
-        }
-        else
-        {
-          const float * P = s_G + 12 * parent;
-          float tl[3] = {s_Jt[3 * j] - s_Jt[3 * parent], s_Jt[3 * j + 1] - s_Jt[3 * parent + 1],
-                         s_Jt[3 * j + 2] - s_Jt[3 * parent + 2]};
-          for(int r = 0; r < 3; r++)
-          {
-            float p0 = P[4 * r], p1 = P[4 * r + 1], p2 = P[4 * r + 2], p3 = P[4 * r + 3];
-            for(int c = 0; c < 3; c++) G[4 * r + c] = p0 * R[c] + p1 * R[3 + c] + p2 * R[6 + c];
-            G[4 * r + 3] = p0 * tl[0] + p1 * tl[1] + p2 * tl[2] + p3;
-          }
-        }
-      }
-      __syncwarp();
-    }
-    if(j < kJoints)
-    {
-      const float * G = s_G + 12 * j;
-      for(int r = 0; r < 3; r++)
-        s_tp[3 * j + r] = G[4 * r + 3] - (G[4 * r] * s_Jt[3 * j] + G[4 * r + 1] * s_Jt[3 * j + 1] + G[4 * r + 2] * s_Jt[3 * j + 2]);
-    }
-  }
+  if(tid < 32) chain_globals_warp(tid, p.topo, s_R, s_Jt, s_G, s_tp);
   __syncthreads();
   // ---- skinning of the task vertices (LinearBlendSkinning.cpp:445-553 on the ~480 rows the tasks touch): the terms
   //      wn_j x_uj = (W[u,j] / sum W) (Rg_j rest_u + t'_j) are what the chain columns need anyway (P5b), their sum over
@@ -296,10 +239,7 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
       const int i = u * t.kmax + sl;
       const int j = s_sj[i];
       const float wj = s_sw[i];
-      const float * G = s_G + 12 * j;
-      const f3 x = mk3(wj * (G[0] * ru.x + G[1] * ru.y + G[2] * ru.z + s_tp[3 * j]),
-                       wj * (G[4] * ru.x + G[5] * ru.y + G[6] * ru.z + s_tp[3 * j + 1]),
-                       wj * (G[8] * ru.x + G[9] * ru.y + G[10] * ru.z + s_tp[3 * j + 2]));
+      const f3 x = skin_term(s_G + 12 * j, s_tp + 3 * j, 1, ru, wj);
       s_xw[3 * i] = x.x, s_xw[3 * i + 1] = x.y, s_xw[3 * i + 2] = x.z;
       acc = acc + x;
     }
@@ -307,27 +247,7 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
     s_verts[3 * u] = v.x, s_verts[3 * u + 1] = v.y, s_verts[3 * u + 2] = v.z;
   }
   // ---- P2b: M_kc = Rg_parent(k) dR_kc Rg_k^T  (d x_j / d theta_kc = M_kc (x_j - tg_k)) ----
-  if(tid < 72)
-  {
-    const int k = tid / 3;
-    const float * A = s_dR + 9 * tid;
-    const float * Rk = s_G + 12 * k;
-    const int parent = p.topo.parent[k];
-    float T[9];
-    if(parent < 0)
-    {
-      for(int e = 0; e < 9; e++) T[e] = A[e];
-    }
-    else
-    {
-      const float * P = s_G + 12 * parent;
-      for(int a = 0; a < 3; a++)
-        for(int e = 0; e < 3; e++) T[3 * a + e] = P[4 * a] * A[e] + P[4 * a + 1] * A[3 + e] + P[4 * a + 2] * A[6 + e];
-    }
-    for(int a = 0; a < 3; a++)
-      for(int b = 0; b < 3; b++)
-        s_M[9 * tid + 3 * a + b] = T[3 * a] * Rk[4 * b] + T[3 * a + 1] * Rk[4 * b + 1] + T[3 * a + 2] * Rk[4 * b + 2];
-  }
+  if(tid < 72) chain_dM(tid, p.topo, s_dR, s_G, s_M);
   // ---- P2c: d tg_j / d beta and d t'_j / d beta (3x10 per joint).  One warp per beta component, lane = joint: the walk down
   //      the tree needs only warp barriers (it was a block barrier per level: a dozen of them with 240 busy threads) ----
   if(p.beta_cols)
@@ -340,32 +260,10 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
     {
       for(int d = 0; d <= p.topo.max_depth; d++)
       {
-        if(on && depth == d)
-        {
-          if(parent < 0)
-          {
-            for(int r = 0; r < 3; r++) s_dTg[(3 * j + r) * kShapeDim + i] = s_JS[(3 * j + r) * kShapeDim + i];
-          }
-          else
-          {
-            const float * P = s_G + 12 * parent;
-            float dl[3];
-            for(int r = 0; r < 3; r++) dl[r] = s_JS[(3 * j + r) * kShapeDim + i] - s_JS[(3 * parent + r) * kShapeDim + i];
-            for(int r = 0; r < 3; r++)
-              s_dTg[(3 * j + r) * kShapeDim + i] =
-                  s_dTg[(3 * parent + r) * kShapeDim + i] + P[4 * r] * dl[0] + P[4 * r + 1] * dl[1] + P[4 * r + 2] * dl[2];
-          }
-        }
+        if(on && depth == d) chain_dtg_dbeta(j, i, parent, s_G, s_JS, s_dTg);
         __syncwarp();
       }
-      if(on)
-      {
-        const float * G = s_G + 12 * j;
-        float js[3] = {s_JS[(3 * j) * kShapeDim + i], s_JS[(3 * j + 1) * kShapeDim + i], s_JS[(3 * j + 2) * kShapeDim + i]};
-        for(int r = 0; r < 3; r++)
-          s_dTp[(3 * j + r) * kShapeDim + i] =
-              s_dTg[(3 * j + r) * kShapeDim + i] - (G[4 * r] * js[0] + G[4 * r + 1] * js[1] + G[4 * r + 2] * js[2]);
-      }
+      if(on) chain_dtp_dbeta(j, i, s_G, s_JS, s_dTg, s_dTp);
     }
   }
   __syncthreads(); // posed vertices complete
@@ -374,10 +272,9 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
   {
     for(int it = tid; it < t.nItems; it += THREADS)
     {
-      f3 v0 = ld3(s_verts + 3 * t.item_verts[3 * it]), v1 = ld3(s_verts + 3 * t.item_verts[3 * it + 1]),
-         v2 = ld3(s_verts + 3 * t.item_verts[3 * it + 2]);
       float inv;
-      f3 nn = normalize_inv(cross3(v1 - v0, v2 - v0), inv);
+      const f3 nn = face_normal(ld3(s_verts + 3 * t.item_verts[3 * it]), ld3(s_verts + 3 * t.item_verts[3 * it + 1]),
+                                ld3(s_verts + 3 * t.item_verts[3 * it + 2]), inv);
       s_itemN[4 * it] = nn.x, s_itemN[4 * it + 1] = nn.y, s_itemN[4 * it + 2] = nn.z, s_itemN[4 * it + 3] = inv;
     }
   }
@@ -387,12 +284,8 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
   {
     for(int ci = tid; ci < 3 * n; ci += THREADS)
     {
-      int s0 = t.item_off[ci], s1 = t.item_off[ci + 1];
-      float wg = 1.f / static_cast<float>(s1 - s0);
-      f3 q = mk3(0.f, 0.f, 0.f);
-      for(int it = s0; it < s1; it++) q = q + wg * ld3(s_itemN + 4 * it);
       float inv;
-      f3 nn = normalize_inv(q, inv);
+      const f3 nn = corner_normal(t.item_off[ci], t.item_off[ci + 1], [&](int it) { return ld3(s_itemN + 4 * it); }, inv);
       s_cornN[4 * ci] = nn.x, s_cornN[4 * ci + 1] = nn.y, s_cornN[4 * ci + 2] = nn.z, s_cornN[4 * ci + 3] = inv;
     }
   }
@@ -408,58 +301,31 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
       v[c] = ld3(s_verts + 3 * t.corner[3 * m + c]);
       nc[c] = p.use_ring ? ld3(s_cornN + 4 * (3 * m + c)) : mk3(0.f, 0.f, 0.f);
     }
-    float w[3] = {p.vertex_weights[3 * fm], p.vertex_weights[3 * fm + 1], p.vertex_weights[3 * fm + 2]};
-    f3 pos = w[0] * v[0] + w[1] * v[1] + w[2] * v[2];
-    float inv_s = 0.f;
-    if(p.use_ring && p.normal_offset > 0.f)
-      pos = pos + p.normal_offset * normalize_inv(w[0] * nc[0] + w[1] * nc[1] + w[2] * nc[2], inv_s);
-    float wn[3];
-    triangle_weights(pos, v[0], v[1], v[2], wn);
+    const float w[3] = {p.vertex_weights[3 * fm], p.vertex_weights[3 * fm + 1], p.vertex_weights[3 * fm + 2]};
+    float wn[3], inv_s;
+    f3 nh;
+    const f3 pos = reweight_task(v, nc, w, p.use_ring, p.normal_offset, wn, nh, inv_s);
     if(p.update_weights)
       p.vertex_weights[3 * fm] = wn[0], p.vertex_weights[3 * fm + 1] = wn[1], p.vertex_weights[3 * fm + 2] = wn[2];
-    f3 nh = mk3(0.f, 0.f, 0.f);
-    if(p.use_ring) nh = normalize_inv(wn[0] * nc[0] + wn[1] * nc[1] + wn[2] * nc[2], inv_s);
-    f3 pn = wn[0] * v[0] + wn[1] * v[1] + wn[2] * v[2];
-    if(p.normal_offset > 0.f) pn = pn + p.normal_offset * nh;
     const float posw = p.pos_task_weight ? p.pos_task_weight[fm] : 1.f;
-    f3 tgt = ld3(p.target_pos + 3 * fm);
-    f3 nt = p.target_normal ? ld3(p.target_normal + 3 * fm) : mk3(0.f, 0.f, 1.f);
-    float e[4] = {posw * (pn.x - tgt.x), posw * (pn.y - tgt.y), posw * (pn.z - tgt.z),
-                  p.normal_task_weight > 0.f ? p.normal_task_weight * (dot3(nh, nt) + 1.f) : 0.f};
+    const f3 tgt = ld3(p.target_pos + 3 * fm);
+    const f3 nt = p.target_normal ? ld3(p.target_normal + 3 * fm) : mk3(0.f, 0.f, 1.f);
+    float e[4];
+    task_residual(v, wn, nh, p.normal_offset, posw, tgt, nt, p.normal_task_weight, e);
     float * eo = p.e_out + static_cast<size_t>(f) * 4 * n + 4 * m;
     eo[0] = e[0], eo[1] = e[1], eo[2] = e[2], eo[3] = e[3];
     if(!(isfinite(e[0]) && isfinite(e[1]) && isfinite(e[2]) && isfinite(e[3]))) atomicOr(&s_bad, 1);
     if(posw > 0.f) atomicAdd(&s_valid, 1);
-    float * ts = s_task + TS * m;
-    ts[0] = wn[0], ts[1] = wn[1], ts[2] = wn[2];
-    ts[3] = nh.x, ts[4] = nh.y, ts[5] = nh.z, ts[6] = inv_s, ts[7] = posw;
-    ts[8] = nt.x, ts[9] = nt.y, ts[10] = nt.z;
+    store_task_scratch(s_task + TS * m, wn, nh, inv_s, posw, nt);
     if(p.phi_cols)
     {
-      // d w' / d pos (pos = detached actual position + tangents phi, IkTask.cpp:49-57), tangents (:33-47)
-      f3 r0 = cross3(v[1] - pos, v[2] - pos), r1 = cross3(v[2] - pos, v[0] - pos), r2 = cross3(v[0] - pos, v[1] - pos);
-      float a0 = norm3(r0), a1 = norm3(r1), a2 = norm3(r2), S = a0 + a1 + a2;
-      f3 g0 = cross3((1.f / a0) * r0, v[2] - v[1]), g1 = cross3((1.f / a1) * r1, v[0] - v[2]),
-         g2 = cross3((1.f / a2) * r2, v[1] - v[0]);
-      f3 gs = g0 + g1 + g2;
-      f3 dw[3] = {(1.f / S) * (g0 - wn[0] * gs), (1.f / S) * (g1 - wn[1] * gs), (1.f / S) * (g2 - wn[2] * gs)};
-      f3 t1 = v[1] - v[0];
-      f3 nrm = cross3(t1, v[2] - v[0]);
-      f3 t2 = cross3(nrm, t1);
-      float dummy;
-      f3 tang[2] = {normalize_inv(t1, dummy), normalize_inv(t2, dummy)};
+      f3 dw[3], tang[2];
+      phi_frame(pos, wn, v, dw, tang);
       for(int k = 0; k < 2; k++)
       {
-        float dwk[3] = {dot3(dw[0], tang[k]), dot3(dw[1], tang[k]), dot3(dw[2], tang[k])};
-        f3 dp = dwk[0] * v[0] + dwk[1] * v[1] + dwk[2] * v[2];
-        f3 dn = mk3(0.f, 0.f, 0.f);
-        if(p.use_ring) dn = proj_apply(nh, inv_s, dwk[0] * nc[0] + dwk[1] * nc[1] + dwk[2] * nc[2]);
-        if(p.normal_offset > 0.f) dp = dp + p.normal_offset * dn;
-        const int col = 75 + 2 * m + k;
-        Jf[(4 * m + 0) * p.ldfull + col] = posw * dp.x;
-        Jf[(4 * m + 1) * p.ldfull + col] = posw * dp.y;
-        Jf[(4 * m + 2) * p.ldfull + col] = posw * dp.z;
-        Jf[(4 * m + 3) * p.ldfull + col] = p.normal_task_weight > 0.f ? p.normal_task_weight * dot3(nt, dn) : 0.f;
+        float col[4];
+        phi_column(dw, tang, k, v, nc, nh, inv_s, p.use_ring, p.normal_offset, posw, nt, p.normal_task_weight, col);
+        for(int r = 0; r < 4; r++) Jf[(4 * m + r) * p.ldfull + 75 + 2 * m + k] = col[r];
       }
     }
   }
@@ -513,14 +379,11 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
         f3 S[3] = {mk3(0.f, 0.f, 0.f), mk3(0.f, 0.f, 0.f), mk3(0.f, 0.f, 0.f)};
         do
         {
-          const int slot = t.pair_refs[rf] & 3;
-          f3 v0 = ld3(s_verts + 3 * t.item_verts[3 * it]), v1 = ld3(s_verts + 3 * t.item_verts[3 * it + 1]),
-             v2 = ld3(s_verts + 3 * t.item_verts[3 * it + 2]);
-          f3 e1 = v1 - v0, e2 = v2 - v0;
-          f3 a = slot == 0 ? (e2 - e1) : (slot == 1 ? mk3(-e2.x, -e2.y, -e2.z) : e1);
+          f3 ax[3];
+          ref_edge_cross(ld3(s_verts + 3 * t.item_verts[3 * it]), ld3(s_verts + 3 * t.item_verts[3 * it + 1]),
+                         ld3(s_verts + 3 * t.item_verts[3 * it + 2]), t.pair_refs[rf] & 3, ax);
           const f3 ng = ld3(s_itemN + 4 * it);
           const float inv_g = s_itemN[4 * it + 3];
-          const f3 ax[3] = {mk3(0.f, a.z, -a.y), mk3(-a.z, 0.f, a.x), mk3(a.y, -a.x, 0.f)}; // a x e_c
 #pragma unroll
           for(int cc = 0; cc < 3; cc++) S[cc] = S[cc] + proj_apply(ng, inv_g, ax[cc]);
           rf++;
@@ -537,22 +400,7 @@ __global__ void __launch_bounds__(TC ? c1::THREADS_TC : c1::THREADS, 2) ik_jacob
         }
       }
     }
-    const float posw = ts[7];
-    const float wc = q < 3 ? ts[q] : 0.f; // pairs 0..2 of a task are its corners 0..2
-#pragma unroll
-    for(int r = 0; r < 3; r++)
-#pragma unroll
-      for(int c = 0; c < 3; c++) C[3 * r + c] = posw * (((r == c) ? wc : 0.f) + p.normal_offset * D[3 * r + c]);
-    if(ROWS == 4)
-    {
-      const float nw = p.normal_task_weight;
-#pragma unroll
-      for(int c = 0; c < 3; c++) C[9 + c] = nw * (ts[8] * D[c] + ts[9] * D[3 + c] + ts[10] * D[6 + c]);
-    }
-    else
-    {
-      C[9] = C[10] = C[11] = 0.f;
-    }
+    c4_block<ROWS>(ts, q, D, p.normal_offset, p.normal_task_weight, C);
   }
   __syncthreads();
   if(tid == 0)
@@ -2139,6 +1987,25 @@ size_t solve_smem_bytes(const IkLayout & L, bool schur)
   return solve_rows_off(L, schur) + 2 * 4 * static_cast<size_t>(L.ld) * sizeof(float) + 16;
 }
 
+// theta (B, 75) fed to the forward pass: the state itself, or [trans | root | decoder(latent) | hands] with the decoder
+// Jacobian on the side (node.cpp:761-772)
+int assemble_theta(const smplpp_vposer_t * vposer, const IkLayout & L, cudaStream_t st, int B, float * theta_state, char * ws,
+                   const float ** theta75, const float ** vjac)
+{
+  *theta75 = theta_state;
+  *vjac = nullptr;
+  if(!L.vposer) return SMPLPP_OK;
+  float * theta = reinterpret_cast<float *>(ws + L.off_theta);
+  float * jac = reinterpret_cast<float *>(ws + L.off_vjac);
+  theta_assemble_kernel<<<(B * 12 + 127) / 128, 128, 0, st>>>(B, theta_state, theta);
+  SB_LAUNCHED();
+  int rc = launch_vposer_decode(vposer, st, B, theta_state + 6, 44, theta + 6, 75, jac, reinterpret_cast<float *>(ws + L.off_vaux));
+  if(rc != SMPLPP_OK) return rc;
+  *theta75 = theta;
+  *vjac = jac;
+  return SMPLPP_OK;
+}
+
 // shared front end of smplpp_ik_step and smplpp_ik_shared_beta_reduce for one chunk of frames
 int run_chunk(const smplpp_model_t * model, const smplpp_vposer_t * vposer, const smplpp_tasks_t * tasks,
               const smplpp_ik_options * o, const IkLayout & L, cudaStream_t st, int B, float * theta_state,
@@ -2146,23 +2013,15 @@ int run_chunk(const smplpp_model_t * model, const smplpp_vposer_t * vposer, cons
               const float * target_normal, const float * pos_task_weight, char * ws)
 {
   const ModelDev & md = model->d;
-  float * theta = reinterpret_cast<float *>(ws + L.off_theta);
   float * coef = reinterpret_cast<float *>(ws + L.off_coef);
   float * xf = reinterpret_cast<float *>(ws + L.off_xf);
   float * verts = reinterpret_cast<float *>(ws + L.off_verts);
   float * rest = reinterpret_cast<float *>(ws + L.off_rest);
-  float * vjac = L.vposer ? reinterpret_cast<float *>(ws + L.off_vjac) : nullptr;
-  const float * theta_in = theta_state;
-  if(L.vposer)
-  {
-    theta_assemble_kernel<<<(B * 12 + 127) / 128, 128, 0, st>>>(B, theta_state, theta);
-    SB_LAUNCHED();
-    int rc = launch_vposer_decode(vposer, st, B, theta_state + 6, 44, theta + 6, 75, vjac,
-                                  reinterpret_cast<float *>(ws + L.off_vaux));
-    if(rc != SMPLPP_OK) return rc;
-    theta_in = theta;
-  }
-  int rc = launch_pose_chain(md, st, B, beta, beta_stride, theta_in, coef, xf, nullptr, nullptr);
+  const float * theta_in;
+  const float * vjac;
+  int rc = assemble_theta(vposer, L, st, B, theta_state, ws, &theta_in, &vjac);
+  if(rc != SMPLPP_OK) return rc;
+  rc = launch_pose_chain(md, st, B, beta, beta_stride, theta_in, coef, xf, nullptr, nullptr);
   if(rc != SMPLPP_OK) return rc;
   const ModelDev & sub = L.use_ring ? tasks->sub : tasks->sub_corner;
   // rest shape of the task vertices: tcgen05 (blocked frame layout) where the task set has the operand images
@@ -2270,6 +2129,21 @@ IkSolveParams make_solve_params(const smplpp_ik_options * o, const IkLayout & L,
   sp.a_ws = L.qp_ws ? reinterpret_cast<double *>(ws + L.off_aws) : nullptr;
   return sp;
 }
+
+// the solve of one chunk: J'J on the fp64 tensor cores where the problem shape allows, else ik_solve_kernel
+int launch_solve(IkSolveParams & sp, const IkLayout & L, bool schur, cudaStream_t st)
+{
+  const size_t smem = solve_smem_bytes(L, schur);
+  sp.rows_off = static_cast<int>(solve_rows_off(L, schur));
+  bool handled = false;
+  const int rc = launch_ik_solve_mma(sp, st, &handled);
+  if(rc != SMPLPP_OK || handled) return rc;
+  if(smem > 227 * 1024) return fail(SMPLPP_ERR_INVALID, "IkTask", "IK problem too large for one CTA per frame");
+  SB_CUDA(cudaFuncSetAttribute(ik_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  ik_solve_kernel<<<sp.B, solve_block_threads(L.D), smem, st>>>(sp);
+  SB_LAUNCHED();
+  return SMPLPP_OK;
+}
 } // namespace
 
 extern "C" size_t smplpp_ik_workspace_bytes(const smplpp_tasks_t * tasks, const smplpp_ik_options * opt, int64_t batch)
@@ -2277,28 +2151,6 @@ extern "C" size_t smplpp_ik_workspace_bytes(const smplpp_tasks_t * tasks, const 
   if(!tasks || !opt || batch < 1) return 0;
   return make_layout(tasks, opt, batch, false).total;
 }
-
-namespace
-{
-// theta (B, 75) fed to the forward pass: the state itself, or [trans | root | decoder(latent) | hands] with the decoder
-// Jacobian on the side (node.cpp:761-772)
-int assemble_theta(const smplpp_vposer_t * vposer, const IkLayout & L, cudaStream_t st, int B, float * theta_state, char * ws,
-                   const float ** theta75, const float ** vjac)
-{
-  *theta75 = theta_state;
-  *vjac = nullptr;
-  if(!L.vposer) return SMPLPP_OK;
-  float * theta = reinterpret_cast<float *>(ws + L.off_theta);
-  float * jac = reinterpret_cast<float *>(ws + L.off_vjac);
-  theta_assemble_kernel<<<(B * 12 + 127) / 128, 128, 0, st>>>(B, theta_state, theta);
-  SB_LAUNCHED();
-  int rc = launch_vposer_decode(vposer, st, B, theta_state + 6, 44, theta + 6, 75, jac, reinterpret_cast<float *>(ws + L.off_vaux));
-  if(rc != SMPLPP_OK) return rc;
-  *theta75 = theta;
-  *vjac = jac;
-  return SMPLPP_OK;
-}
-} // namespace
 
 // face_idx (B, n) int32, nullable: per-frame IkTask::faceIdx_ (re-seated by smplpp_ik_reproject); records_ws: B * n records
 static int ik_step_impl(const smplpp_model_t * model, const smplpp_vposer_t * vposer, const smplpp_tasks_t * tasks,
@@ -2389,16 +2241,8 @@ static int ik_step_impl(const smplpp_model_t * model, const smplpp_vposer_t * vp
     sp.a_out = a_out ? a_out + s * L.dim_ref * L.dim_ref : nullptr;
     sp.b_out = b_out ? b_out + s * L.dim_ref : nullptr;
     sp.delta_out = delta_out ? delta_out + s * L.dim_ref : nullptr;
-    const size_t smem = solve_smem_bytes(L, false);
-    sp.rows_off = static_cast<int>(solve_rows_off(L, false));
-    bool handled = false;
-    rc = launch_ik_solve_mma(sp, st, &handled); // J'J on the fp64 tensor cores where the problem shape allows
+    rc = launch_solve(sp, L, false, st);
     if(rc != SMPLPP_OK) return rc;
-    if(handled) continue;
-    if(smem > 227 * 1024) return fail(SMPLPP_ERR_INVALID, "IkTask", "IK problem too large for one CTA per frame");
-    SB_CUDA(cudaFuncSetAttribute(ik_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    ik_solve_kernel<<<B, solve_block_threads(L.D), smem, st>>>(sp);
-    SB_LAUNCHED();
   }
   return SMPLPP_OK;
 }
@@ -2589,15 +2433,8 @@ extern "C" int smplpp_ik_shared_beta_reduce(const smplpp_model_t * model, const 
     sp.status = status + s;
     sp.schur_out = reinterpret_cast<double *>(ws + L.off_schur) + s * 111;
     sp.factor_ws = reinterpret_cast<double *>(ws + L.off_factor) + s * P;
-    const size_t smem = solve_smem_bytes(L, true);
-    sp.rows_off = static_cast<int>(solve_rows_off(L, true));
-    bool handled = false;
-    rc = launch_ik_solve_mma(sp, st, &handled);
+    rc = launch_solve(sp, L, true, st);
     if(rc != SMPLPP_OK) return rc;
-    if(handled) continue;
-    SB_CUDA(cudaFuncSetAttribute(ik_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    ik_solve_kernel<<<B, solve_block_threads(L.D), smem, st>>>(sp);
-    SB_LAUNCHED();
   }
   schur_reduce_kernel<<<111, 256, 0, st>>>(static_cast<int>(batch), reinterpret_cast<const double *>(ws + L.off_schur), reduced);
   SB_LAUNCHED();

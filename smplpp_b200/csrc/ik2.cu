@@ -517,24 +517,7 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
   for(int i = tt; i < NT * 16; i += TEAM) s_A[i] = 0.0;
   for(int i = tt; i < p.Dp + 4; i += TEAM) s_b[i] = 0.0;
   team_sync(team);
-  if(tt < kJoints)
-  {
-    const int j = tt;
-    rodrigues_grad(s_theta[3 + 3 * j], s_theta[4 + 3 * j], s_theta[5 + 3 * j], s_R + 9 * j, s_dR + 27 * j);
-#pragma unroll
-    for(int k = 0; k < 3; k++)
-    {
-      float acc = p.joint_template[3 * j + k];
-#pragma unroll
-      for(int i = 0; i < kShapeDim; i++)
-      {
-        const float js = p.joint_shape[(3 * j + k) * kShapeDim + i];
-        acc = fmaf(js, s_beta[i], acc);
-        if(p.beta_cols) s_JS[(3 * j + k) * kShapeDim + i] = js;
-      }
-      s_Jt[3 * j + k] = acc;
-    }
-  }
+  if(tt < kJoints) chain_joint(tt, s_theta, s_beta, p.joint_template, p.joint_shape, p.beta_cols, s_R, s_dR, s_Jt, s_JS);
   team_sync(team);
   // blend coefficients of the frame: pose feature vec(R_1..R_23) - vec(I) | beta | 0 ...  The template column (217) is
   // NOT part of the dot product: the ~1 m template is added last, to the fully reduced sum of the mm-sized blend terms
@@ -551,70 +534,9 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
       v = s_beta[i - kPoseDim];
     s_coef[i] = v;
   }
-  if(tt < 32)
-  {
-    const int j = tt;
-    const int parent = j < kJoints ? p.topo.parent[j] : -1;
-    const int depth = j < kJoints ? p.topo.depth[j] : -1;
-    for(int d = 0; d <= p.topo.max_depth; d++)
-    {
-      if(depth == d)
-      {
-        const float * Rj = s_R + 9 * j;
-        float * G = s_G + 12 * j;
-        if(parent < 0)
-        {
-          for(int r = 0; r < 3; r++)
-          {
-            G[4 * r] = Rj[3 * r], G[4 * r + 1] = Rj[3 * r + 1], G[4 * r + 2] = Rj[3 * r + 2];
-            G[4 * r + 3] = s_Jt[3 * j + r];
-          }
-        }
-        else
-        {
-          const float * P = s_G + 12 * parent;
-          const float tl[3] = {s_Jt[3 * j] - s_Jt[3 * parent], s_Jt[3 * j + 1] - s_Jt[3 * parent + 1],
-                               s_Jt[3 * j + 2] - s_Jt[3 * parent + 2]};
-          for(int r = 0; r < 3; r++)
-          {
-            const float p0 = P[4 * r], p1 = P[4 * r + 1], p2 = P[4 * r + 2], p3 = P[4 * r + 3];
-            for(int c = 0; c < 3; c++) G[4 * r + c] = p0 * Rj[c] + p1 * Rj[3 + c] + p2 * Rj[6 + c];
-            G[4 * r + 3] = p0 * tl[0] + p1 * tl[1] + p2 * tl[2] + p3;
-          }
-        }
-      }
-      __syncwarp();
-    }
-    if(j < kJoints)
-    {
-      const float * G = s_G + 12 * j;
-      for(int r = 0; r < 3; r++)
-        s_tp[3 * j + r] = G[4 * r + 3] - (G[4 * r] * s_Jt[3 * j] + G[4 * r + 1] * s_Jt[3 * j + 1] + G[4 * r + 2] * s_Jt[3 * j + 2]);
-    }
-  }
+  if(tt < 32) chain_globals_warp(tt, p.topo, s_R, s_Jt, s_G, s_tp);
   team_sync(team);
-  // M_kc = Rg_parent(k) dR_kc Rg_k^T  (d x_j / d theta_kc = M_kc (x_j - tg_k))
-  if(tt < 72)
-  {
-    const int k = tt / 3;
-    const float * Ad = s_dR + 9 * tt;
-    const float * Rk = s_G + 12 * k;
-    const int parent = p.topo.parent[k];
-    float T[9];
-    if(parent < 0)
-    {
-      for(int e = 0; e < 9; e++) T[e] = Ad[e];
-    }
-    else
-    {
-      const float * P = s_G + 12 * parent;
-      for(int a = 0; a < 3; a++)
-        for(int e = 0; e < 3; e++) T[3 * a + e] = P[4 * a] * Ad[e] + P[4 * a + 1] * Ad[3 + e] + P[4 * a + 2] * Ad[6 + e];
-    }
-    for(int a = 0; a < 3; a++)
-      for(int b = 0; b < 3; b++)
-        s_M[9 * tt + 3 * a + b] = T[3 * a] * Rk[4 * b] + T[3 * a + 1] * Rk[4 * b + 1] + T[3 * a + 2] * Rk[4 * b + 2];
-  }
+  if(tt < 72) chain_dM(tt, p.topo, s_dR, s_G, s_M);
   // d tg_j / d beta and d t'_j / d beta (3 x 10 per joint)
   if(p.beta_cols)
   {
@@ -623,33 +545,11 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
       for(int u = tt; u < kJoints * kShapeDim; u += TEAM)
       {
         const int j = u / kShapeDim, i = u % kShapeDim;
-        if(p.topo.depth[j] != d) continue;
-        const int parent = p.topo.parent[j];
-        if(parent < 0)
-        {
-          for(int r = 0; r < 3; r++) s_dTg[(3 * j + r) * kShapeDim + i] = s_JS[(3 * j + r) * kShapeDim + i];
-        }
-        else
-        {
-          const float * P = s_G + 12 * parent;
-          float dl[3];
-          for(int r = 0; r < 3; r++) dl[r] = s_JS[(3 * j + r) * kShapeDim + i] - s_JS[(3 * parent + r) * kShapeDim + i];
-          for(int r = 0; r < 3; r++)
-            s_dTg[(3 * j + r) * kShapeDim + i] =
-                s_dTg[(3 * parent + r) * kShapeDim + i] + P[4 * r] * dl[0] + P[4 * r + 1] * dl[1] + P[4 * r + 2] * dl[2];
-        }
+        if(p.topo.depth[j] == d) chain_dtg_dbeta(j, i, p.topo.parent[j], s_G, s_JS, s_dTg);
       }
       team_sync(team);
     }
-    for(int u = tt; u < kJoints * kShapeDim; u += TEAM)
-    {
-      const int j = u / kShapeDim, i = u % kShapeDim;
-      const float * G = s_G + 12 * j;
-      const float js[3] = {s_JS[(3 * j) * kShapeDim + i], s_JS[(3 * j + 1) * kShapeDim + i], s_JS[(3 * j + 2) * kShapeDim + i]};
-      for(int r = 0; r < 3; r++)
-        s_dTp[(3 * j + r) * kShapeDim + i] =
-            s_dTg[(3 * j + r) * kShapeDim + i] - (G[4 * r] * js[0] + G[4 * r + 1] * js[1] + G[4 * r + 2] * js[2]);
-    }
+    for(int u = tt; u < kJoints * kShapeDim; u += TEAM) chain_dtp_dbeta(u / kShapeDim, u % kShapeDim, s_G, s_JS, s_dTg, s_dTp);
   }
   team_sync(team);
 
@@ -770,9 +670,8 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
         s_sw[i] = wj;
         s_sj[i] = static_cast<uint8_t>(j);
         const float * G = s_G + 12 * j;
-        s_xw[3 * i] = wj * (G[0] * ru.x + G[1] * ru.y + G[2] * ru.z + s_tp[3 * j]);
-        s_xw[3 * i + 1] = wj * (G[4] * ru.x + G[5] * ru.y + G[6] * ru.z + s_tp[3 * j + 1]);
-        s_xw[3 * i + 2] = wj * (G[8] * ru.x + G[9] * ru.y + G[10] * ru.z + s_tp[3 * j + 2]);
+        const f3 x = skin_term(G, s_tp + 3 * j, 1, ru, wj);
+        s_xw[3 * i] = x.x, s_xw[3 * i + 1] = x.y, s_xw[3 * i + 2] = x.z;
 #pragma unroll
         for(int r = 0; r < 3; r++)
         {
@@ -818,9 +717,8 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
       for(int it0 = tt; it0 < nie; it0 += 32)
       {
         const uint8_t * it = s_rec->item[it0];
-        const f3 v0 = ld3(s_pv + 3 * it[0]), v1 = ld3(s_pv + 3 * it[1]), v2 = ld3(s_pv + 3 * it[2]);
         float inv;
-        const f3 nn = normalize_inv(cross3(v1 - v0, v2 - v0), inv);
+        const f3 nn = face_normal(ld3(s_pv + 3 * it[0]), ld3(s_pv + 3 * it[1]), ld3(s_pv + 3 * it[2]), inv);
         s_itemN[4 * it0] = nn.x, s_itemN[4 * it0 + 1] = nn.y, s_itemN[4 * it0 + 2] = nn.z, s_itemN[4 * it0 + 3] = inv;
       }
       __syncwarp(); // items, corners and the task are chained inside warp 0
@@ -828,12 +726,8 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
       {
         int s0 = 0;
         for(int c = 0; c < tt; c++) s0 += s_rec->nic[c];
-        const int cnt = s_rec->nic[tt];
-        const float wg = 1.f / static_cast<float>(cnt);
-        f3 q = mk3(0.f, 0.f, 0.f);
-        for(int it = s0; it < s0 + cnt; it++) q = q + wg * ld3(s_itemN + 4 * it);
         float inv;
-        const f3 nn = normalize_inv(q, inv);
+        const f3 nn = corner_normal(s0, s0 + s_rec->nic[tt], [&](int it) { return ld3(s_itemN + 4 * it); }, inv);
         s_cornN[4 * tt] = nn.x, s_cornN[4 * tt + 1] = nn.y, s_cornN[4 * tt + 2] = nn.z, s_cornN[4 * tt + 3] = inv;
       }
       __syncwarp();
@@ -847,6 +741,8 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
         v[c] = rec_ok ? ld3(s_pv + 3 * c) : mk3(0.f, 0.f, 0.f);
         nc[c] = p.use_ring ? ld3(s_cornN + 4 * c) : mk3(0.f, 0.f, 0.f);
       }
+      // reweight_task, task_residual, store_task_scratch, phi_frame / phi_column (ik_math.cuh) written inline: through the
+      // helpers ptxas spills 4-12 more bytes in this kernel
       const float w[3] = {s_tin[3 * m], s_tin[3 * m + 1], s_tin[3 * m + 2]};
       f3 pos = w[0] * v[0] + w[1] * v[1] + w[2] * v[2];
       float inv_s = 0.f;
@@ -923,12 +819,10 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
         const float scale = s_ts[c] * wg;
         const f3 nh = mk3(s_ts[3], s_ts[4], s_ts[5]);
         const float inv_s = s_ts[6];
-        const f3 v0 = ld3(s_pv + 3 * iv[0]), v1 = ld3(s_pv + 3 * iv[1]), v2 = ld3(s_pv + 3 * iv[2]);
-        const f3 e1 = v1 - v0, e2 = v2 - v0;
-        const f3 a = slot == 0 ? (e2 - e1) : (slot == 1 ? mk3(-e2.x, -e2.y, -e2.z) : e1);
+        f3 ax[3];
+        ref_edge_cross(ld3(s_pv + 3 * iv[0]), ld3(s_pv + 3 * iv[1]), ld3(s_pv + 3 * iv[2]), slot, ax);
         const f3 ng = ld3(s_itemN + 4 * it), nci = ld3(s_cornN + 4 * c);
         const float inv_g = s_itemN[4 * it + 3], inv_q = s_cornN[4 * c + 3];
-        const f3 ax[3] = {mk3(0.f, a.z, -a.y), mk3(-a.z, 0.f, a.x), mk3(a.y, -a.x, 0.f)}; // a x e_c
         float * D = s_Dref + 9 * tt;
 #pragma unroll
         for(int cc = 0; cc < 3; cc++)
@@ -954,21 +848,8 @@ __global__ void __launch_bounds__(k2::MAXF * k2::TEAM + 32, 1) ik_fused_kernel(c
           for(int e = 0; e < 9; e++) D[e] += Dr[e];
         }
       }
-      const float posw = s_ts[7];
-      const float wc = tt < 3 ? s_ts[tt] : 0.f;
       float * C = s_C4 + 12 * tt;
-#pragma unroll
-      for(int r = 0; r < 3; r++)
-#pragma unroll
-        for(int c = 0; c < 3; c++) C[3 * r + c] = posw * (((r == c) ? wc : 0.f) + p.normal_offset * D[3 * r + c]);
-      if(ROWS == 4)
-      {
-        const float nw = p.normal_task_weight;
-#pragma unroll
-        for(int c = 0; c < 3; c++) C[9 + c] = nw * (s_ts[8] * D[c] + s_ts[9] * D[3 + c] + s_ts[10] * D[6 + c]);
-      }
-      else
-        C[9] = C[10] = C[11] = 0.f;
+      c4_block<ROWS>(s_ts, tt, D, p.normal_offset, p.normal_task_weight, C);
       // CA4 = C4 . A_u (the pose-blend columns contract it with the basis rows)
       const float * Au = s_Au + 9 * tt;
       float * CA = s_CA4 + 12 * tt;

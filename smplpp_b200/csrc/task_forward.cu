@@ -58,9 +58,10 @@ size_t points_smem_bytes(const TasksDev & t, int nUse, bool use_ring)
 }
 } // namespace
 
-// One CTA per frame.  The arithmetic is that of task_positions_kernel (ik.cu) and of the skinning block of
-// ik_jacobian_kernel: homogeneous weights W / sum W (any number of influences), uniform 1 / deg weights of the 1-ring
-// face normals, normalize_inv everywhere.
+// One CTA per frame.  Skinning, face and corner normals are skin_term, face_normal and corner_normal of ik_math.cuh
+// (homogeneous weights W / sum W, any number of influences).  calcActualPos stays written out here and in
+// task_positions_kernel: through one shared helper that takes the corners by callable, the normals of this kernel came
+// out different in the last bits.
 __global__ void __launch_bounds__(kPointsThreads) task_points_kernel(const TaskPointsParams p)
 {
   extern __shared__ __align__(16) float sm[];
@@ -91,10 +92,7 @@ __global__ void __launch_bounds__(kPointsThreads) task_points_kernel(const TaskP
       const int j = __ldg(t.sj_flat + i);
       const float wj = __ldg(t.sw_norm + i);
       const float * G = s_xf + kXformFloats * j;
-      const f3 x = mk3(wj * (G[0] * ru.x + G[1] * ru.y + G[2] * ru.z + G[3]),
-                       wj * (G[4] * ru.x + G[5] * ru.y + G[6] * ru.z + G[7]),
-                       wj * (G[8] * ru.x + G[9] * ru.y + G[10] * ru.z + G[11]));
-      acc = acc + x;
+      acc = acc + skin_term(G, G + 3, 4, ru, wj);
     }
     v = v + acc;
     s_verts[3 * u] = v.x, s_verts[3 * u + 1] = v.y, s_verts[3 * u + 2] = v.z;
@@ -105,22 +103,18 @@ __global__ void __launch_bounds__(kPointsThreads) task_points_kernel(const TaskP
     // ---- face normals of the 1-ring items (SMPL::calcNormal) ----
     for(int it = tid; it < t.nItems; it += kPointsThreads)
     {
-      const f3 a = ld3(s_verts + 3 * __ldg(t.item_verts + 3 * it)), b = ld3(s_verts + 3 * __ldg(t.item_verts + 3 * it + 1)),
-               c = ld3(s_verts + 3 * __ldg(t.item_verts + 3 * it + 2));
       float inv;
-      const f3 nn = normalize_inv(cross3(b - a, c - a), inv);
+      const f3 nn = face_normal(ld3(s_verts + 3 * __ldg(t.item_verts + 3 * it)), ld3(s_verts + 3 * __ldg(t.item_verts + 3 * it + 1)),
+                                ld3(s_verts + 3 * __ldg(t.item_verts + 3 * it + 2)), inv);
       s_itemN[3 * it] = nn.x, s_itemN[3 * it + 1] = nn.y, s_itemN[3 * it + 2] = nn.z;
     }
     __syncthreads();
-    // ---- vertex normals of the corners (SMPL::calcVertexNormal, src/SMPL.cpp:527-535) ----
+    // ---- vertex normals of the corners (SMPL::calcVertexNormal) ----
     for(int ci = tid; ci < 3 * t.n; ci += kPointsThreads)
     {
-      const int s0 = __ldg(t.item_off + ci), s1 = __ldg(t.item_off + ci + 1);
-      const float wg = 1.f / static_cast<float>(s1 - s0);
-      f3 q = mk3(0.f, 0.f, 0.f);
-      for(int it = s0; it < s1; it++) q = q + wg * ld3(s_itemN + 3 * it);
       float inv;
-      const f3 nn = normalize_inv(q, inv);
+      const f3 nn = corner_normal(__ldg(t.item_off + ci), __ldg(t.item_off + ci + 1), [&](int it) { return ld3(s_itemN + 3 * it); },
+                                  inv);
       s_cornN[3 * ci] = nn.x, s_cornN[3 * ci + 1] = nn.y, s_cornN[3 * ci + 2] = nn.z;
     }
     __syncthreads();
